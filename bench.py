@@ -7,6 +7,7 @@ LSQR and CRAIG advanced in lock-step by the fused two-column SpMM kernels.
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one rank per GPU)
     python bench.py --impl reference --steps K --warmup W    # CPU arm: the oracle port on host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also writes the last timed step's outputs as .npy
 
 value : whole-job solves/s with rhs / Jacobian values already resident in HBM (FPSB_DEVICE)
 e2e   : the same step through the C ABI with HOST buffers (FPSB_HOST: jac values + both rhs
@@ -33,6 +34,26 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 SQRT_EPS = float(np.sqrt(np.finfo(np.float64).eps))
+
+OUTPUT_NAMES = ("p1", "q1", "p2", "q2")
+STAT_FIELDS = ("niter", "solved", "inconsistent", "status", "rnorm", "arnorm", "anorm", "acond", "xnorm")
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(d, out):
+    """--dump-outputs: what one solve_two_mixed call returns, as DIR/<name>.npy in float64 — the four solution
+    vectors p1, q1, p2, q2 and stats.npy, the LSQR and CRAIG stats as a (2, 9) array in STAT_FIELDS order.  At the
+    default size the vectors take 24 MB and are written whole; past 64 MB every vector is cut to the same share of
+    its entries at positions drawn from a fixed seed, so two runs of the same arguments write the same positions."""
+    vecs = [x.cpu().numpy().astype(np.float64) for x in out[:4]]
+    total = sum(v.nbytes for v in vecs)
+    os.makedirs(d, exist_ok=True)
+    for name, v in zip(OUTPUT_NAMES, vecs):
+        if total > DUMP_LIMIT_BYTES:
+            keep = len(v) * (DUMP_LIMIT_BYTES - 4096) // total
+            v = v[np.sort(np.random.default_rng(0).choice(len(v), keep, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), v)
+    np.save(os.path.join(d, "stats.npy"), np.array([[float(s[f]) for f in STAT_FIELDS] for s in out[4]]))
 
 
 def make_workload(n, m, k, w, seed):
@@ -425,7 +446,13 @@ def main():
     ap.add_argument("--no-partitioned", action="store_true", help="N>1: skip the strong-scaled row-partitioned record")
     ap.add_argument("--part-grid", type=int, default=2048, help="grid of the C3 operator of the partitioned record")
     ap.add_argument("--part-iters", type=int, default=100, help="fixed Krylov iterations of the C3 partitioned run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) to DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
 
     n, m, k, w = args.n, args.m, args.nnz_per_row, args.window
     cfg = {"workload": "C4-shape synthetic sparse equality-constrained problem: window-random Jacobian "
@@ -504,6 +531,7 @@ def main():
     barrier()
     clocks = sampler.stop()
     launches = H.launch_count() - l0
+    last_out = out
     st = out[4]
     t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -780,6 +808,8 @@ def main():
     }
     if partitioned is not None:
         line["partitioned"] = partitioned
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_out)
     print(json.dumps(line))
 
 

@@ -52,6 +52,7 @@ EXPORTS = [
     "fpsb_ldlt_analyze", "fpsb_ldlt_symbolic_sizes", "fpsb_ldlt_get_symbolic",
     "fpsb_ldlt_plan_info", "fpsb_ldlt_factorize", "fpsb_ldlt_get_factor",
     "fpsb_ldlt_solve_two_mixed", "fpsb_ldlt_solve_two_least_squares", "fpsb_ldlt_solve_two_extras",
+    "fpsb_ldlt_batch_solve_two_mixed", "fpsb_ldlt_batch_solve_two_least_squares",
     "fpsb_symbolic_create", "fpsb_symbolic_destroy", "fpsb_symbolic_sizes", "fpsb_symbolic_get",
     "fpsb_symbolic_plan_info", "fpsb_order_dissection", "fpsb_batch_solve_two",
     "fpsb_dist_unique_id", "fpsb_dist_attach", "fpsb_dist_jprod", "fpsb_dist_jtprod",

@@ -35,8 +35,9 @@ constexpr int kTrsmRows = 2 * kUpdRows;                 // rows of L21 staged pe
 constexpr int kFacDoubles = kBS * kMaxW + 2 * kMaxW + 2 * kUpdRows * kMaxW;      // B | dd | rk | S | C
 constexpr int kSolveRows = 1024;                        // rows of a panel whose x[R[r]] are staged per pass of the backward solve
 constexpr int kSolDoubles = kBS * kMaxW + 2 * kMaxW + 2 * kSolveRows + 2 * kWarpsPerBlock * kMaxW;   // L11 | ys | xr | per-warp partials
-static_assert(kSmallW * (kSmallW + 1) + 4 * kSmallW <= kFacDoubles / kWarpsPerBlock, "warp-level supernodes share the block's buffer");
-static_assert(kSmallW * (kSmallW + 1) + 4 * kSmallW <= kSolDoubles / kWarpsPerBlock, "warp-level supernodes share the block's buffer");
+constexpr int kWarpShDoubles = (kSmallW + 1) * kSmallW + 4 * kSmallW;   // per warp-level supernode
+static_assert(kWarpShDoubles <= kFacDoubles / kWarpsPerBlock, "warp-level supernodes share the block's buffer");
+static_assert(kWarpShDoubles <= kSolDoubles / kWarpsPerBlock, "warp-level supernodes share the block's buffer");
 
 struct PlanDev {
     int N, nsuper, ntasks;
@@ -70,6 +71,17 @@ struct PlanDev {
     int dynamic_reg;
     unsigned long long *tstamp;   // debug builds (-DFPSB_LDLT_TIMERS): [3][nsuper] completion times (globaltimer ns)
 };
+// The storage one numeric factorisation works on: the handle's own (single instance, SYNC routines: flags and
+// tickets order the supernodes across CTAs) or one instance's slice of the batched factor store (one CTA owns the
+// instance and walks the plan level by level: no flags, __syncthreads between dependent steps).
+struct LdltWork {
+    double *panels;
+    double *D;
+    double2 *Y;
+    int *fail;
+};
+__host__ __device__ __forceinline__ LdltWork work_of(const PlanDev &P) { return LdltWork{P.panels, P.D, P.Y, P.fail}; }
+
 #ifdef FPSB_LDLT_TIMERS
 #define LDLT_STAMP(P, phase, t) do { unsigned long long now_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now_)); \
         (P).tstamp[(size_t)(phase) * (P).nsuper + (t)] = now_; } while (0)
@@ -88,6 +100,17 @@ struct LdltPlan {
     DevBuf<double2> Y;
     DevBuf<int> done_f, done_s, done_b, ticket, fail;
     DevBuf<unsigned long long> tstamp;
+    // batched path: supernodes grouped into steps of mutually independent ones (bsn; bstep: {first, first warp-level,
+    // end} per step, step 0 = the leaves wider than one column, step l = dependency level l), the factor store
+    // (ninst x bstride doubles: panels | D), per-CTA right-hand sides, per-instance factorisation status
+    DevBuf<int> bsn, bstep;
+    int nbstep = 0;
+    int64_t bstride = 0;
+    DevBuf<double> bstore;
+    DevBuf<double2> bY;
+    DevBuf<int> bok;
+    int64_t bstore_inst = 0, bY_rows = 0, bok_inst = 0;
+    int64_t bninst = -1;        // ninst of the last batched mixed call (-1: none), whose factors bstore holds
     int ntasks = 0;
     int epoch = 0;
     int64_t naslot = 0;
@@ -138,10 +161,8 @@ __device__ __forceinline__ void wait_done(const int *flag, int epoch, int tid, i
 // ------------------------------------------------------------------------------------------------
 // assembly: panels <- [1..1 | jac values | -delta..]  through the precomputed slot map
 // ------------------------------------------------------------------------------------------------
-__global__ void assemble_kernel(int64_t nslot, const int64_t *aslot, const int64_t *aptr, const int *asrc,
-                                const double *jvals, int nvar, int64_t nnzj, double delta, double *panels) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nslot) return;
+__device__ __forceinline__ void assemble_slot(int64_t i, const int64_t *aslot, const int64_t *aptr, const int *asrc,
+                                              const double *jvals, int nvar, int64_t nnzj, double delta, double *panels) {
     double s = 0.0;
     for (int64_t p = aptr[i]; p < aptr[i + 1]; ++p) {
         int id = asrc[p];
@@ -150,29 +171,35 @@ __global__ void assemble_kernel(int64_t nslot, const int64_t *aslot, const int64
     }
     panels[aslot[i]] = s;
 }
+__global__ void assemble_kernel(int64_t nslot, const int64_t *aslot, const int64_t *aptr, const int *asrc,
+                                const double *jvals, int nvar, int64_t nnzj, double delta, double *panels) {
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nslot) return;
+    assemble_slot(i, aslot, aptr, asrc, jvals, nvar, nnzj, delta, panels);
+}
 
 // ------------------------------------------------------------------------------------------------
 // numeric factorisation of one supernode (left-looking)
 // ------------------------------------------------------------------------------------------------
-template <bool WARP>
-__device__ void factor_supernode(const PlanDev &P, int t, double *sh, int epoch, int tid, int nt) {
+template <bool WARP, bool SYNC = true>
+__device__ void factor_supernode(const PlanDev &P, const LdltWork &W, int t, double *sh, int epoch, int tid, int nt) {
     const int f = P.sfirst[t];
     const int w = P.sfirst[t + 1] - f;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
     const int ld = w + nr;
-    double *panel = P.panels + P.poff[t];
+    double *panel = W.panels + P.poff[t];
 
     // 1. pull the updates of every non-leaf descendant supernode (leaf contributions were applied
     //    by leaf_update_kernel before this launch)
     for (int64_t q = P.uptr[t]; q < P.umid[t]; ++q) {
         const int d = P.usrc[q];
-        wait_done<WARP>(&P.done_f[d], epoch, tid, P.fail);
+        if (SYNC) wait_done<WARP>(&P.done_f[d], epoch, tid, P.fail);
         const int fd = P.sfirst[d];
         const int wd = P.sfirst[d + 1] - fd;
         const int nrd = (int)(P.rptr[d + 1] - P.rptr[d]);
         const int ldd = wd + nrd;
-        const double *pd = P.panels + P.poff[d] + wd;     // rows below d's block
-        const double *Dd = P.D + fd;
+        const double *pd = W.panels + P.poff[d] + wd;     // rows below d's block
+        const double *Dd = W.D + fd;
         const int a = P.ua[q], b = P.ub[q];
         const int *relq = P.rel + P.urel[q];
         const int nrow = nrd - a, ncol = b - a;
@@ -210,9 +237,9 @@ __device__ void factor_supernode(const PlanDev &P, int t, double *sh, int epoch,
                 const double sg = (double)((r > 0.0) - (r < 0.0));
                 dk = sg * fmax(fabs(dk + r), fabs(r));
             }
-            if (dk == 0.0) { atomicCAS(P.fail, 0, f + k + 1); dk = 1.0; }
+            if (dk == 0.0) { atomicCAS(W.fail, 0, f + k + 1); dk = 1.0; }
             dd[k] = dk;
-            P.D[f + k] = dk;
+            W.D[f + k] = dk;
         }
         gsync<WARP>();
         const double dk = dd[k];
@@ -247,36 +274,36 @@ __device__ void factor_supernode(const PlanDev &P, int t, double *sh, int epoch,
             row[(size_t)k * ld] = s / dd[k];
         }
     }
-    __threadfence();
+    if (SYNC) __threadfence();
     gsync<WARP>();
-    if (tid == 0) { st_release(&P.done_f[t], epoch); LDLT_STAMP(P, 0, t); }
+    if (SYNC && tid == 0) { st_release(&P.done_f[t], epoch); LDLT_STAMP(P, 0, t); }
 }
 
-template <bool WARP>
-__device__ void fwd_supernode(const PlanDev &P, int t, double *sh, int epoch, int tid, int nt) {
+template <bool WARP, bool SYNC = true>
+__device__ void fwd_supernode(const PlanDev &P, const LdltWork &W, int t, double *sh, int epoch, int tid, int nt) {
     const int f = P.sfirst[t];
     const int w = P.sfirst[t + 1] - f;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
     const int ld = w + nr;
-    const double *panel = P.panels + P.poff[t];
+    const double *panel = W.panels + P.poff[t];
     double2 *ys = reinterpret_cast<double2 *>(sh);     // w entries
-    for (int k = tid; k < w; k += nt) ys[k] = P.Y[f + k];
+    for (int k = tid; k < w; k += nt) ys[k] = W.Y[f + k];
     gsync<WARP>();
     for (int64_t q = P.uptr[t]; q < P.umid[t]; ++q) {
         const int d = P.usrc[q];
-        wait_done<WARP>(&P.done_s[d], epoch, tid, P.fail);
+        if (SYNC) wait_done<WARP>(&P.done_s[d], epoch, tid, P.fail);
         const int fd = P.sfirst[d];
         const int wd = P.sfirst[d + 1] - fd;
         const int nrd = (int)(P.rptr[d + 1] - P.rptr[d]);
         const int ldd = wd + nrd;
-        const double *pd = P.panels + P.poff[d] + wd;
+        const double *pd = W.panels + P.poff[d] + wd;
         const int a = P.ua[q], b = P.ub[q];
         const int *relq = P.rel + P.urel[q];
         for (int j = a + tid; j < b; j += nt) {
             double s0 = 0.0, s1 = 0.0;
             for (int k = 0; k < wd; ++k) {
                 const double l = __ldcg(pd + (size_t)k * ldd + j);
-                const double2 yv = __ldcg(P.Y + fd + k);
+                const double2 yv = __ldcg(W.Y + fd + k);
                 s0 += l * yv.x; s1 += l * yv.y;
             }
             const int lc = relq[j - a];
@@ -293,21 +320,21 @@ __device__ void fwd_supernode(const PlanDev &P, int t, double *sh, int epoch, in
         }
         gsync<WARP>();
     }
-    for (int k = tid; k < w; k += nt) P.Y[f + k] = ys[k];
-    __threadfence();
+    for (int k = tid; k < w; k += nt) W.Y[f + k] = ys[k];
+    if (SYNC) __threadfence();
     gsync<WARP>();
-    if (tid == 0) { st_release(&P.done_s[t], epoch); LDLT_STAMP(P, 1, t); }
+    if (SYNC && tid == 0) { st_release(&P.done_s[t], epoch); LDLT_STAMP(P, 1, t); }
 }
 
-template <bool WARP>
-__device__ void bwd_supernode(const PlanDev &P, int t, double *sh, int epoch, int tid, int nt, bool nowait) {
+template <bool WARP, bool SYNC = true>
+__device__ void bwd_supernode(const PlanDev &P, const LdltWork &W, int t, double *sh, int epoch, int tid, int nt, bool nowait) {
     const int f = P.sfirst[t];
     const int w = P.sfirst[t + 1] - f;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
     const int ld = w + nr;
-    const double *panel = P.panels + P.poff[t];
+    const double *panel = W.panels + P.poff[t];
     const int *R = P.rows + P.rptr[t];
-    if (!nowait)
+    if (SYNC && !nowait)
         for (int64_t q = P.tptr[t]; q < P.tptr[t + 1]; ++q)
             wait_done<WARP>(&P.done_b[P.ttgt[q]], epoch, tid, P.fail);
     double2 *xs = reinterpret_cast<double2 *>(sh);     // w entries
@@ -318,13 +345,13 @@ __device__ void bwd_supernode(const PlanDev &P, int t, double *sh, int epoch, in
         const double *col = panel + (size_t)k * ld + w;
         for (int r = lane; r < nr; r += 32) {
             const double l = col[r];
-            const double2 xv = __ldcg(P.Y + R[r]);
+            const double2 xv = __ldcg(W.Y + R[r]);
             s0 += l * xv.x; s1 += l * xv.y;
         }
         s0 = warp_sum(s0); s1 = warp_sum(s1);
         if (lane == 0) {
-            const double2 yv = P.Y[f + k];
-            const double dk = P.D[f + k];
+            const double2 yv = W.Y[f + k];
+            const double dk = W.D[f + k];
             xs[k] = make_double2(yv.x / dk - s0, yv.y / dk - s1);
         }
     }
@@ -337,10 +364,10 @@ __device__ void bwd_supernode(const PlanDev &P, int t, double *sh, int epoch, in
         }
         gsync<WARP>();
     }
-    for (int k = tid; k < w; k += nt) P.Y[f + k] = xs[k];
-    __threadfence();
+    for (int k = tid; k < w; k += nt) W.Y[f + k] = xs[k];
+    if (SYNC) __threadfence();
     gsync<WARP>();
-    if (tid == 0) { st_release(&P.done_b[t], epoch); LDLT_STAMP(P, 2, t); }
+    if (SYNC && tid == 0) { st_release(&P.done_b[t], epoch); LDLT_STAMP(P, 2, t); }
 }
 
 
@@ -366,16 +393,16 @@ __device__ __forceinline__ void dmma_m8n8k4(double &c0, double &c1, double a, do
 // pass, C: the b - a "column rows" scaled by D), each thread owns a 4 x 4 register tile (rows ti + 16 ii, columns
 // 4 tj + jj), or, with DMMA, each warp owns 8 x 64 strips of 8 x 8 tensor-core tiles.
 template <bool DMMA>
-__device__ __forceinline__ void schur_update_block(const PlanDev &P, int64_t q, double *panel, int ld, double *S, double *Cc,
-                                                   int tid) {
+__device__ __forceinline__ void schur_update_block(const PlanDev &P, const LdltWork &W, int64_t q, double *panel, int ld,
+                                                   double *S, double *Cc, int tid) {
     const int d = P.usrc[q];
     const int fd = P.sfirst[d];
     const int wd = P.sfirst[d + 1] - fd;
     const int nrd = (int)(P.rptr[d + 1] - P.rptr[d]);
     const int ldd = wd + nrd;
     const int a = P.ua[q], b = P.ub[q];
-    const double *pd = P.panels + P.poff[d] + wd + a;     // row a of the rows below d's block
-    const double *Dd = P.D + fd;
+    const double *pd = W.panels + P.poff[d] + wd + a;     // row a of the rows below d's block
+    const double *Dd = W.D + fd;
     const int *relq = P.rel + P.urel[q];
     const int nrow = nrd - a, ncol = b - a;
     for (int e = tid; e < wd * kUpdRows; e += kLdltBlock) {
@@ -456,14 +483,14 @@ __device__ __forceinline__ void schur_update_block(const PlanDev &P, int64_t q, 
     }
 }
 
-template <bool DMMA>
-__device__ void factor_supernode_block(const PlanDev &P, int t, double *sh, int epoch, int tid) {
+template <bool DMMA, bool SYNC = true>
+__device__ void factor_supernode_block(const PlanDev &P, const LdltWork &W, int t, double *sh, int epoch, int tid) {
     constexpr int nt = kLdltBlock;
     const int f = P.sfirst[t];
     const int w = P.sfirst[t + 1] - f;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
     const int ld = w + nr;
-    double *panel = P.panels + P.poff[t];
+    double *panel = W.panels + P.poff[t];
     double *B = sh;                          // [w][kBS] lower triangle, row-major
     double *dd = B + kBS * kMaxW;            // pivots
     double *rk = dd + kMaxW;                 // regularisation value of each pivot
@@ -472,8 +499,8 @@ __device__ void factor_supernode_block(const PlanDev &P, int t, double *sh, int 
 
     // 1. updates of every non-leaf descendant (leaf contributions were applied by leaf_update_kernel before)
     for (int64_t q = P.uptr[t]; q < P.umid[t]; ++q) {
-        wait_done<false>(&P.done_f[P.usrc[q]], epoch, tid, P.fail);
-        schur_update_block<DMMA>(P, q, panel, ld, S, Cc, tid);
+        if (SYNC) wait_done<false>(&P.done_f[P.usrc[q]], epoch, tid, P.fail);
+        schur_update_block<DMMA>(P, W, q, panel, ld, S, Cc, tid);
     }
     __syncthreads();
 
@@ -494,7 +521,7 @@ __device__ void factor_supernode_block(const PlanDev &P, int t, double *sh, int 
         }
         const bool zero = (dk == 0.0);
         if (zero) dk = 1.0;
-        if (tid == 0) { dd[k] = dk; if (zero) atomicCAS(P.fail, 0, f + k + 1); }
+        if (tid == 0) { dd[k] = dk; if (zero) atomicCAS(W.fail, 0, f + k + 1); }
         const int i = k + 1 + (tid >> 2);
         if (i < w) {
             const double lik = B[i * kBS + k] / dk;
@@ -502,7 +529,7 @@ __device__ void factor_supernode_block(const PlanDev &P, int t, double *sh, int 
         }
         __syncthreads();
     }
-    if (tid < w) P.D[f + tid] = dd[tid];
+    if (tid < w) W.D[f + tid] = dd[tid];
     for (int e = tid; e < w * w; e += nt) {
         const int j = e / w, i = e - j * w;
         if (i > j) {
@@ -541,9 +568,11 @@ __device__ void factor_supernode_block(const PlanDev &P, int t, double *sh, int 
         }
         __syncthreads();
     }
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) { st_release(&P.done_f[t], epoch); LDLT_STAMP(P, 0, t); }
+    if (SYNC) {
+        __threadfence();
+        __syncthreads();
+        if (tid == 0) { st_release(&P.done_f[t], epoch); LDLT_STAMP(P, 0, t); }
+    }
 }
 
 // 2-column forward / backward substitution with the w x w unit triangle held in shared memory (forward: k-major,
@@ -573,13 +602,14 @@ __device__ __forceinline__ void tri_solve_warp(const double *Ls, double2 *ys, in
     if (lane + 32 < w) ys[lane + 32] = y1;
 }
 
-__device__ void fwd_supernode_block(const PlanDev &P, int t, double *sh, int epoch, int tid) {
+template <bool SYNC = true>
+__device__ void fwd_supernode_block(const PlanDev &P, const LdltWork &W, int t, double *sh, int epoch, int tid) {
     constexpr int nt = kLdltBlock;
     const int f = P.sfirst[t];
     const int w = P.sfirst[t + 1] - f;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
     const int ld = w + nr;
-    const double *panel = P.panels + P.poff[t];
+    const double *panel = W.panels + P.poff[t];
     double *Ls = sh;                                                    // [w][64] k-major strict lower triangle
     double2 *ys = reinterpret_cast<double2 *>(sh + kBS * kMaxW);      // w entries
     double2 *part = ys + kMaxW + kSolveRows;                            // [8 warps][w] partial pulls
@@ -596,19 +626,19 @@ __device__ void fwd_supernode_block(const PlanDev &P, int t, double *sh, int epo
     double2 *mine = part + wid * kMaxW;
     for (int64_t q = P.uptr[t] + wid; q < P.umid[t]; q += kWarpsPerBlock) {
         const int d = P.usrc[q];
-        wait_done<true>(&P.done_s[d], epoch, lane, P.fail);
+        if (SYNC) wait_done<true>(&P.done_s[d], epoch, lane, P.fail);
         const int fd = P.sfirst[d];
         const int wd = P.sfirst[d + 1] - fd;
         const int nrd = (int)(P.rptr[d + 1] - P.rptr[d]);
         const int ldd = wd + nrd;
-        const double *pd = P.panels + P.poff[d] + wd;
+        const double *pd = W.panels + P.poff[d] + wd;
         const int a = P.ua[q], b = P.ub[q];
         const int *relq = P.rel + P.urel[q];
         for (int j = a + lane; j < b; j += 32) {
             double s0 = 0.0, s1 = 0.0;
             for (int k = 0; k < wd; ++k) {
                 const double l = __ldcg(pd + (size_t)k * ldd + j);
-                const double2 yv = __ldcg(P.Y + fd + k);
+                const double2 yv = __ldcg(W.Y + fd + k);
                 s0 += l * yv.x; s1 += l * yv.y;
             }
             const int lc = relq[j - a];
@@ -618,7 +648,7 @@ __device__ void fwd_supernode_block(const PlanDev &P, int t, double *sh, int epo
     }
     __syncthreads();
     for (int k = tid; k < w; k += nt) {
-        double2 y = P.Y[f + k];
+        double2 y = W.Y[f + k];
 #pragma unroll
         for (int u = 0; u < kWarpsPerBlock; ++u) { const double2 pp = part[u * kMaxW + k]; y.x -= pp.x; y.y -= pp.y; }
         ys[k] = y;
@@ -627,20 +657,23 @@ __device__ void fwd_supernode_block(const PlanDev &P, int t, double *sh, int epo
     if (wid == 0) {
         tri_solve_warp(Ls, ys, w, lane, false);
         __syncwarp();
-        for (int k = lane; k < w; k += 32) P.Y[f + k] = ys[k];
-        __threadfence();
-        __syncwarp();
-        if (lane == 0) { st_release(&P.done_s[t], epoch); LDLT_STAMP(P, 1, t); }
+        for (int k = lane; k < w; k += 32) W.Y[f + k] = ys[k];
+        if (SYNC) {
+            __threadfence();
+            __syncwarp();
+            if (lane == 0) { st_release(&P.done_s[t], epoch); LDLT_STAMP(P, 1, t); }
+        }
     }
 }
 
-__device__ void bwd_supernode_block(const PlanDev &P, int t, double *sh, int epoch, int tid, bool nowait) {
+template <bool SYNC = true>
+__device__ void bwd_supernode_block(const PlanDev &P, const LdltWork &W, int t, double *sh, int epoch, int tid, bool nowait) {
     constexpr int nt = kLdltBlock;
     const int f = P.sfirst[t];
     const int w = P.sfirst[t + 1] - f;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
     const int ld = w + nr;
-    const double *panel = P.panels + P.poff[t];
+    const double *panel = W.panels + P.poff[t];
     const int *R = P.rows + P.rptr[t];
     double *Ls = sh;                                                    // [i][kBS] row-major: Ls[i*kBS + k] = L(i, k)
     double2 *xs = reinterpret_cast<double2 *>(sh + kBS * kMaxW);      // w entries
@@ -651,19 +684,19 @@ __device__ void bwd_supernode_block(const PlanDev &P, int t, double *sh, int epo
         if (i > k) Ls[i * kBS + k] = panel[(size_t)k * ld + i];
     }
     prefetch_l2_range(panel, (size_t)ld * w, tid, nt);
-    if (!nowait)
+    if (SYNC && !nowait)
         for (int64_t q = P.tptr[t]; q < P.tptr[t + 1]; ++q)
             wait_done<false>(&P.done_b[P.ttgt[q]], epoch, tid, P.fail);
     // xs[k] = y_k / d_k - sum_r L21[r][k] x[R[r]] : the gathered x are staged once, a warp per column
     for (int k = tid; k < w; k += nt) {
-        const double2 yv = P.Y[f + k];
-        const double dk = P.D[f + k];
+        const double2 yv = W.Y[f + k];
+        const double dk = W.D[f + k];
         xs[k] = make_double2(yv.x / dk, yv.y / dk);
     }
     for (int r0 = 0; r0 < nr; r0 += kSolveRows) {
         const int rows = min(kSolveRows, nr - r0);
         __syncthreads();
-        for (int r = tid; r < rows; r += nt) xr[r] = __ldcg(P.Y + R[r0 + r]);
+        for (int r = tid; r < rows; r += nt) xr[r] = __ldcg(W.Y + R[r0 + r]);
         __syncthreads();
         for (int k = wid; k < w; k += kWarpsPerBlock) {
             double s0 = 0.0, s1 = 0.0;
@@ -681,10 +714,12 @@ __device__ void bwd_supernode_block(const PlanDev &P, int t, double *sh, int epo
     if (wid == 0) {
         tri_solve_warp(Ls, xs, w, lane, true);
         __syncwarp();
-        for (int k = lane; k < w; k += 32) P.Y[f + k] = xs[k];
-        __threadfence();
-        __syncwarp();
-        if (lane == 0) { st_release(&P.done_b[t], epoch); LDLT_STAMP(P, 2, t); }
+        for (int k = lane; k < w; k += 32) W.Y[f + k] = xs[k];
+        if (SYNC) {
+            __threadfence();
+            __syncwarp();
+            if (lane == 0) { st_release(&P.done_b[t], epoch); LDLT_STAMP(P, 2, t); }
+        }
     }
 }
 
@@ -699,6 +734,7 @@ __global__ void __launch_bounds__(kLdltBlock, MODE == 0 ? 4 : 2) ldlt_phase_kern
     extern __shared__ __align__(16) double sh[];
     __shared__ int s_task;
     const int tid = threadIdx.x;
+    const LdltWork W = work_of(P);
     for (;;) {
         if (tid == 0) s_task = atomicAdd(&P.ticket[tk], 1);
         __syncthreads();
@@ -710,23 +746,23 @@ __global__ void __launch_bounds__(kLdltBlock, MODE == 0 ? 4 : 2) ldlt_phase_kern
         if (cnt == 0) {
             const int t = P.order[t0];
             if (MODE == 0) {
-                if (PHASE == 0) factor_supernode<false>(P, t, sh, epoch, tid, kLdltBlock);
-                else if (PHASE == 1) fwd_supernode<false>(P, t, sh, epoch, tid, kLdltBlock);
-                else bwd_supernode<false>(P, t, sh, epoch, tid, kLdltBlock, nowait != 0);
+                if (PHASE == 0) factor_supernode<false>(P, W, t, sh, epoch, tid, kLdltBlock);
+                else if (PHASE == 1) fwd_supernode<false>(P, W, t, sh, epoch, tid, kLdltBlock);
+                else bwd_supernode<false>(P, W, t, sh, epoch, tid, kLdltBlock, nowait != 0);
             } else {
-                if (PHASE == 0) factor_supernode_block<MODE == 2>(P, t, sh, epoch, tid);
-                else if (PHASE == 1) fwd_supernode_block(P, t, sh, epoch, tid);
-                else bwd_supernode_block(P, t, sh, epoch, tid, nowait != 0);
+                if (PHASE == 0) factor_supernode_block<MODE == 2>(P, W, t, sh, epoch, tid);
+                else if (PHASE == 1) fwd_supernode_block(P, W, t, sh, epoch, tid);
+                else bwd_supernode_block(P, W, t, sh, epoch, tid, nowait != 0);
             }
         } else {
             const int wid = tid >> 5, lane = tid & 31;
             if (wid < cnt) {
                 // in the backward phase the bundle is walked in reverse as well
                 const int t = P.order[PHASE == 2 ? t0 + cnt - 1 - wid : t0 + wid];
-                double *wsh = sh + wid * ((kSmallW + 1) * kSmallW + 4 * kSmallW);
-                if (PHASE == 0) factor_supernode<true>(P, t, wsh, epoch, lane, 32);
-                else if (PHASE == 1) fwd_supernode<true>(P, t, wsh, epoch, lane, 32);
-                else bwd_supernode<true>(P, t, wsh, epoch, lane, 32, nowait != 0);
+                double *wsh = sh + wid * kWarpShDoubles;
+                if (PHASE == 0) factor_supernode<true>(P, W, t, wsh, epoch, lane, 32);
+                else if (PHASE == 1) fwd_supernode<true>(P, W, t, wsh, epoch, lane, 32);
+                else bwd_supernode<true>(P, W, t, wsh, epoch, lane, 32, nowait != 0);
             }
         }
         __syncthreads();
@@ -771,9 +807,8 @@ static void launch_phase(Handle *h, const PlanDev &P, int ntasks, int epoch, int
 // leaf contributions: embarrassingly parallel over TARGET columns (each column is owned by one
 // 8-lane group, sources applied in ascending order => deterministic, no floating-point atomics)
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) leaf_update_kernel(PlanDev P) {
-    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int j = gt >> 3, l8 = gt & 7;
+// column j, lane l8 of the 8-lane group that owns it
+__device__ __forceinline__ void leaf_update_column(const PlanDev &P, const LdltWork &W, int j, int l8) {
     if (j >= P.N) return;
     const int64_t e0 = P.lcptr[j], e1 = P.lcptr[j + 1];
     if (e0 == e1) return;
@@ -781,11 +816,11 @@ __global__ void __launch_bounds__(256) leaf_update_kernel(PlanDev P) {
     const int t = P.sn_of[j];
     const int ft = P.sfirst[t];
     const int ldt = P.sfirst[t + 1] - ft + (int)(P.rptr[t + 1] - P.rptr[t]);
-    double *col = P.panels + P.poff[t] + (size_t)(j - ft) * ldt;
+    double *col = W.panels + P.poff[t] + (size_t)(j - ft) * ldt;
     for (int64_t e = e0; e < e1; ++e) {
-        const double *src = P.panels + P.lc_src[e];
+        const double *src = W.panels + P.lc_src[e];
         const int cnt = P.lc_cnt[e], ldd = P.lc_ldd[e], wd = P.lc_wd[e];
-        const double *Dd = P.D + P.lc_fd[e];
+        const double *Dd = W.D + P.lc_fd[e];
         const int *relp = P.rel + P.lc_rel[e];
         for (int i = l8; i < cnt; i += 8) {
             double s = 0.0;
@@ -795,104 +830,246 @@ __global__ void __launch_bounds__(256) leaf_update_kernel(PlanDev P) {
         __syncwarp(gmask);
     }
 }
+__global__ void __launch_bounds__(256) leaf_update_kernel(PlanDev P) {
+    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
+    leaf_update_column(P, work_of(P), gt >> 3, gt & 7);
+}
 
 // ------------------------------------------------------------------------------------------------
 // one-wide leaf supernodes (a variable nobody was eliminated before: ~2/3 of all columns of a KKT matrix under a
 // dissection ordering).  No dependencies, no triangle: flat kernels, 8 lanes per leaf, instead of tickets and bundles.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) leaf1_factor_kernel(PlanDev P, int nleaf) {
-    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = gt >> 3, l8 = gt & 7;
+__device__ __forceinline__ void leaf1_factor(const PlanDev &P, const LdltWork &W, int i, int l8, int nleaf) {
     if (i >= nleaf) return;
     const int t = P.order[i];
     const int f = P.sfirst[t];
     if (P.sfirst[t + 1] - f != 1) return;
     const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
-    double *panel = P.panels + P.poff[t];
+    double *panel = W.panels + P.poff[t];
     double dk = panel[0];
     if (P.dynamic_reg && fabs(dk) < P.tol) {
         const double r = (P.P[f] < P.n_d) ? P.r1 : P.r2;
         const double sg = (double)((r > 0.0) - (r < 0.0));
         dk = sg * fmax(fabs(dk + r), fabs(r));
     }
-    if (dk == 0.0) { if (l8 == 0) atomicCAS(P.fail, 0, f + 1); dk = 1.0; }
-    if (l8 == 0) P.D[f] = dk;
+    if (dk == 0.0) { if (l8 == 0) atomicCAS(W.fail, 0, f + 1); dk = 1.0; }
+    if (l8 == 0) W.D[f] = dk;
     for (int r = l8; r < nr; r += 8) panel[1 + r] = panel[1 + r] / dk;
 }
-// backward: x_f = y_f / d_f - sum_r L21[r] x[R[r]]  (the rows R are ancestors: already final)
-__global__ void __launch_bounds__(256) leaf1_bwd_kernel(PlanDev P, int nleaf) {
+__global__ void __launch_bounds__(256) leaf1_factor_kernel(PlanDev P, int nleaf) {
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = gt >> 3, l8 = gt & 7;
+    leaf1_factor(P, work_of(P), gt >> 3, gt & 7, nleaf);
+}
+// backward: x_f = y_f / d_f - sum_r L21[r] x[R[r]]  (the rows R are ancestors: already final).  All 32 lanes of the
+// warp call it (8-lane shuffle reduction).
+__device__ __forceinline__ void leaf1_bwd(const PlanDev &P, const LdltWork &W, int i, int l8, int nleaf) {
     const int t = i < nleaf ? P.order[i] : -1;
     const int f = t >= 0 ? P.sfirst[t] : 0;
     const bool on = t >= 0 && P.sfirst[t + 1] - f == 1;
     double s0 = 0.0, s1 = 0.0;
     if (on) {
         const int nr = (int)(P.rptr[t + 1] - P.rptr[t]);
-        const double *col = P.panels + P.poff[t] + 1;
+        const double *col = W.panels + P.poff[t] + 1;
         const int *R = P.rows + P.rptr[t];
         for (int r = l8; r < nr; r += 8) {
             const double l = col[r];
-            const double2 xv = P.Y[R[r]];
+            const double2 xv = W.Y[R[r]];
             s0 += l * xv.x; s1 += l * xv.y;
         }
     }
 #pragma unroll
     for (int o = 4; o > 0; o >>= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); }
     if (on && l8 == 0) {
-        const double2 yv = P.Y[f];
-        const double dk = P.D[f];
-        P.Y[f] = make_double2(yv.x / dk - s0, yv.y / dk - s1);
+        const double2 yv = W.Y[f];
+        const double dk = W.D[f];
+        W.Y[f] = make_double2(yv.x / dk - s0, yv.y / dk - s1);
     }
+}
+__global__ void __launch_bounds__(256) leaf1_bwd_kernel(PlanDev P, int nleaf) {
+    const int gt = blockIdx.x * blockDim.x + threadIdx.x;
+    leaf1_bwd(P, work_of(P), gt >> 3, gt & 7, nleaf);
 }
 
 // forward solve: y[j] -= sum over leaf sources d containing row j of L_d(j, :) . y_d
-__global__ void __launch_bounds__(256) leaf_fwd_update_kernel(PlanDev P) {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+__device__ __forceinline__ void leaf_fwd_update_row(const PlanDev &P, const LdltWork &W, int j) {
     if (j >= P.N) return;
     const int64_t e0 = P.lcptr[j], e1 = P.lcptr[j + 1];
     if (e0 == e1) return;
     double s0 = 0.0, s1 = 0.0;
     for (int64_t e = e0; e < e1; ++e) {
-        const double *src = P.panels + P.lc_src[e];
+        const double *src = W.panels + P.lc_src[e];
         const int ldd = P.lc_ldd[e], wd = P.lc_wd[e], fd = P.lc_fd[e];
         for (int k = 0; k < wd; ++k) {
             const double l = src[(size_t)k * ldd];
-            const double2 yv = P.Y[fd + k];
+            const double2 yv = W.Y[fd + k];
             s0 += l * yv.x; s1 += l * yv.y;
         }
     }
-    double2 y = P.Y[j];
+    double2 y = W.Y[j];
     y.x -= s0; y.y -= s1;
-    P.Y[j] = y;
+    W.Y[j] = y;
+}
+__global__ void __launch_bounds__(256) leaf_fwd_update_kernel(PlanDev P) {
+    leaf_fwd_update_row(P, work_of(P), blockIdx.x * blockDim.x + threadIdx.x);
 }
 
 // Y[k] = (B0[P[k]], B1[P[k]]) with B0 = [rhs1; 0], B1 = kind == 0 ? [0; rhs2] : [rhs2; 0]
-__global__ void load_rhs_kernel(int N, int nvar, int kind, const int *P, const double *rhs1,
-                                const double *rhs2, double2 *Y) {
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= N) return;
+__device__ __forceinline__ double2 rhs_entry(int k, int nvar, int kind, const int *P, const double *rhs1, const double *rhs2) {
     const int i = P[k];
     double2 v;
     v.x = (i < nvar) ? rhs1[i] : 0.0;
     if (kind == 0) v.y = (i < nvar) ? 0.0 : rhs2[i - nvar];
     else v.y = (i < nvar) ? rhs2[i] : 0.0;
-    Y[k] = v;
+    return v;
+}
+__global__ void load_rhs_kernel(int N, int nvar, int kind, const int *P, const double *rhs1,
+                                const double *rhs2, double2 *Y) {
+    int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= N) return;
+    Y[k] = rhs_entry(k, nvar, kind, P, rhs1, rhs2);
+}
+__device__ __forceinline__ void store_sol_entry(int i, int nvar, const int *pinv, const double2 *Y, double *p1, double *q1,
+                                                double *p2, double *q2) {
+    const double2 v = Y[pinv[i]];
+    if (i < nvar) { p1[i] = v.x; p2[i] = v.y; }
+    else { q1[i - nvar] = v.x; q2[i - nvar] = v.y; }
 }
 __global__ void store_sol_kernel(int N, int nvar, const int *pinv, const double2 *Y, double *p1, double *q1,
                                  double *p2, double *q2) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
-    const double2 v = Y[pinv[i]];
-    if (i < nvar) { p1[i] = v.x; p2[i] = v.y; }
-    else { q1[i - nvar] = v.x; q2[i - nvar] = v.y; }
+    store_sol_entry(i, nvar, pinv, Y, p1, q1, p2, q2);
 }
 // reference behaviour on a failed factorisation: `sol` still holds the right-hand sides
-__global__ void passthrough_kernel(int nvar, int ncon, int kind, const double *rhs1, const double *rhs2,
-                                   double *p1, double *q1, double *p2, double *q2) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
+__device__ __forceinline__ void passthrough_entry(int i, int nvar, int ncon, int kind, const double *rhs1, const double *rhs2,
+                                                  double *p1, double *q1, double *p2, double *q2) {
     if (i < nvar) { p1[i] = rhs1[i]; p2[i] = (kind == 0) ? 0.0 : rhs2[i]; }
     if (i < ncon) { q1[i] = 0.0; q2[i] = (kind == 0) ? rhs2[i] : 0.0; }
+}
+__global__ void passthrough_kernel(int nvar, int ncon, int kind, const double *rhs1, const double *rhs2,
+                                   double *p1, double *q1, double *p2, double *q2) {
+    passthrough_entry(blockIdx.x * blockDim.x + threadIdx.x, nvar, ncon, kind, rhs1, rhs2, p1, q1, p2, q2);
+}
+
+// ================================================================================================
+// batched path: many instances of one plan (same pattern and symbolic analysis, their own values, delta and
+// right-hand sides) in one launch.  One CTA owns one instance at a time (i = blockIdx.x, += gridDim.x) and walks the
+// plan in steps of mutually independent supernodes (LdltPlan::bstep) with the routine the single-instance launches
+// pick for each supernode, so every entry goes through the same operations in the same order as there; a
+// __syncthreads between dependent steps is the only synchronisation (no tickets, no flags, no waits).
+// ================================================================================================
+struct BatchDev {
+    const int *sn, *step;       // LdltPlan::bsn / bstep
+    int nstep, nleaf;
+    int64_t ninst, stride, psize;
+    const int64_t *aslot, *aptr;
+    const int *asrc;
+    int64_t naslot, nnzj;
+    const int *pinv;
+    double *store;              // [ninst][stride]: panels | D
+    double2 *Y;                 // [gridDim.x][N]
+    int *ok;                    // [ninst]: factorisation status, kept for the least-squares call
+    const double *jvals, *delta, *rhs1, *rhs2;
+    double *p1, *q1, *p2, *q2;
+    int *factorized;
+    int kind;                   // 0 mixed: refactor + solve ; 1 least squares: solve with the stored factors
+};
+
+// one step: its CTA-level supernodes one after the other, then its warp-level ones spread over the warps.  M: the
+// routines of that part of the plan (0 for the leaves, as their launches; ldlt_mode() for the rest); PHASE 0 factor,
+// 1 forward, 2 backward
+template <int M, int PHASE>
+__device__ __forceinline__ void batch_step(const PlanDev &P, const LdltWork &W, const BatchDev &B, int s, double *sh, int tid) {
+    const int s0 = B.step[3 * s], s1 = B.step[3 * s + 1], s2 = B.step[3 * s + 2];
+    for (int k = s0; k < s1; ++k) {
+        const int t = B.sn[k];
+        if (M == 0) {
+            if (PHASE == 0) factor_supernode<false, false>(P, W, t, sh, 0, tid, kLdltBlock);
+            else if (PHASE == 1) fwd_supernode<false, false>(P, W, t, sh, 0, tid, kLdltBlock);
+            else bwd_supernode<false, false>(P, W, t, sh, 0, tid, kLdltBlock, true);
+        } else {
+            if (PHASE == 0) factor_supernode_block<M == 2, false>(P, W, t, sh, 0, tid);
+            else if (PHASE == 1) fwd_supernode_block<false>(P, W, t, sh, 0, tid);
+            else bwd_supernode_block<false>(P, W, t, sh, 0, tid, true);
+        }
+        __syncthreads();
+    }
+    const int wid = tid >> 5, lane = tid & 31;
+    double *wsh = sh + wid * kWarpShDoubles;
+    for (int k = s1 + wid; k < s2; k += kWarpsPerBlock) {
+        const int t = B.sn[k];
+        if (PHASE == 0) factor_supernode<true, false>(P, W, t, wsh, 0, lane, 32);
+        else if (PHASE == 1) fwd_supernode<true, false>(P, W, t, wsh, 0, lane, 32);
+        else bwd_supernode<true, false>(P, W, t, wsh, 0, lane, 32, true);
+    }
+    __syncthreads();
+}
+
+constexpr int kBatchDoubles = kFacDoubles;     // dynamic shared memory of the batch kernel: the largest routine's
+static_assert(kBatchDoubles >= kSolDoubles && kBatchDoubles >= kShDoubles && kBatchDoubles >= kWarpsPerBlock * kWarpShDoubles,
+              "the batch kernel runs every routine in one buffer");
+
+// MODE: ldlt_mode() (the routines of the non-leaf supernodes); the sequence per instance is that of ldlt_factorize /
+// ldlt_solve2: assemble, one-wide leaves, other leaves, leaf contributions, levels 1.. ; forward, backward, store
+template <int MODE>
+__global__ void __launch_bounds__(kLdltBlock, 2) ldlt_batch_kernel(PlanDev P, BatchDev B) {
+    extern __shared__ __align__(16) double sh[];
+    __shared__ int s_fail;
+    const int tid = threadIdx.x;
+    const int N = P.N, nvar = P.n_d, ncon = P.N - P.n_d;
+    const int n2 = B.kind == 0 ? ncon : nvar;
+    constexpr int kGroups = kLdltBlock / 8;      // 8-lane groups of the leaf routines
+    LdltWork W;
+    W.Y = B.Y + (size_t)blockIdx.x * N;
+    W.fail = &s_fail;
+    for (int64_t i = blockIdx.x; i < B.ninst; i += gridDim.x) {
+        W.panels = B.store + i * B.stride;
+        W.D = W.panels + B.psize;
+        int ok;
+        if (B.kind == 0) {
+            if (tid == 0) s_fail = 0;
+            for (int64_t e = tid; e < B.psize; e += kLdltBlock) W.panels[e] = 0.0;
+            __syncthreads();
+            const double *jv = B.jvals + i * B.nnzj;
+            const double delta = B.delta[i];
+            for (int64_t e = tid; e < B.naslot; e += kLdltBlock)
+                assemble_slot(e, B.aslot, B.aptr, B.asrc, jv, nvar, B.nnzj, delta, W.panels);
+            __syncthreads();
+            for (int l0 = 0; l0 < B.nleaf; l0 += kGroups) leaf1_factor(P, W, l0 + (tid >> 3), tid & 7, B.nleaf);
+            __syncthreads();
+            if (B.nstep > 0) batch_step<0, 0>(P, W, B, 0, sh, tid);
+            if (B.nstep > 1) {
+                for (int j0 = 0; j0 < N; j0 += kGroups) leaf_update_column(P, W, j0 + (tid >> 3), tid & 7);
+                __syncthreads();
+                for (int s = 1; s < B.nstep; ++s) batch_step<MODE, 0>(P, W, B, s, sh, tid);
+            }
+            ok = s_fail == 0;
+            if (tid == 0) B.ok[i] = ok;
+        } else {
+            ok = B.ok[i];
+        }
+        if (tid == 0) B.factorized[i] = ok;
+        const double *r1 = B.rhs1 + i * nvar, *r2 = B.rhs2 + i * n2;
+        double *p1 = B.p1 + i * nvar, *q1 = B.q1 + i * ncon, *p2 = B.p2 + i * nvar, *q2 = B.q2 + i * ncon;
+        if (ok) {
+            for (int k = tid; k < N; k += kLdltBlock) W.Y[k] = rhs_entry(k, nvar, B.kind, P.P, r1, r2);
+            __syncthreads();
+            if (B.nstep > 0) batch_step<0, 1>(P, W, B, 0, sh, tid);
+            if (B.nstep > 1) {
+                for (int j = tid; j < N; j += kLdltBlock) leaf_fwd_update_row(P, W, j);
+                __syncthreads();
+                for (int s = 1; s < B.nstep; ++s) batch_step<MODE, 1>(P, W, B, s, sh, tid);
+                for (int s = B.nstep - 1; s >= 1; --s) batch_step<MODE, 2>(P, W, B, s, sh, tid);
+            }
+            if (B.nstep > 0) batch_step<0, 2>(P, W, B, 0, sh, tid);
+            for (int l0 = 0; l0 < B.nleaf; l0 += kGroups) leaf1_bwd(P, W, l0 + (tid >> 3), tid & 7, B.nleaf);
+            __syncthreads();
+            for (int k = tid; k < N; k += kLdltBlock) store_sol_entry(k, nvar, B.pinv, W.Y, p1, q1, p2, q2);
+        } else {
+            for (int k = tid; k < max(nvar, ncon); k += kLdltBlock) passthrough_entry(k, nvar, ncon, B.kind, r1, r2, p1, q1, p2, q2);
+        }
+        __syncthreads();
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -947,7 +1124,36 @@ void ldlt_analyze(Handle *h, const int64_t *Puser, const fpsb_ldlt_opts *opts) {
         }
     }
     L->ntasks = (int)tstart.size();
+    // batched path: one step per dependency level (supernodes of one level do not depend on each other), the CTA-level
+    // supernodes of a step first; the one-wide leaves are left to leaf1_factor / leaf1_bwd as in the launches above
+    std::vector<int> bsn, bstep;
+    {
+        auto warp_level = [&](int t) {
+            const int w = S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t];
+            const int nr = (int)(S.rptr[(size_t)t + 1] - S.rptr[(size_t)t]);
+            return w <= kSmallW && (int64_t)w * (w + nr) <= 512;
+        };
+        int i = 0;
+        for (int lv = 0; lv < S.nlevels; ++lv) {
+            int j = i;
+            while (j < S.nsuper && S.level[(size_t)S.order[(size_t)j]] == lv) j++;
+            bstep.push_back((int)bsn.size());
+            for (int pass = 0; pass < 2; ++pass) {
+                if (pass == 1) bstep.push_back((int)bsn.size());
+                for (int k = i; k < j; ++k) {
+                    const int t = S.order[(size_t)k];
+                    if (lv == 0 && S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t] == 1) continue;
+                    if (warp_level(t) == (pass == 1)) bsn.push_back(t);
+                }
+            }
+            bstep.push_back((int)bsn.size());
+            i = j;
+        }
+        L->nbstep = S.nlevels;
+        L->bstride = (S.panel_size + S.N + 15) / 16 * 16;
+    }
     cudaStream_t s = h->stream;
+    up(L->bsn, bsn, s); up(L->bstep, bstep, s);
     up(L->sfirst, S.sfirst, s); up(L->rows, S.rows, s); up(L->order, S.order, s);
     up(L->task_start, tstart, s); up(L->task_cnt, tcnt, s);
     up(L->usrc, S.usrc, s); up(L->ua, S.ua, s); up(L->ub, S.ub, s); up(L->rel, S.rel, s);
@@ -1066,6 +1272,58 @@ void ldlt_solve2(Handle *h, int kind, const double *rhs1, const double *rhs2, do
     store_sol_kernel<<<grid, 256, 0, s>>>(N, nvar, L->pinv.p, L->Y.p, p1, q1, p2, q2);
     h->launches += 2;
     FPSB_CUDA(cudaGetLastError());
+}
+
+template <int MODE>
+static void launch_batch(Handle *h, const PlanDev &P, BatchDev &B) {
+    LdltPlan *L = h->ldlt;
+    const size_t smem = (size_t)kBatchDoubles * sizeof(double);
+    FPSB_CUDA(cudaFuncSetAttribute(ldlt_batch_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    FPSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ldlt_batch_kernel<MODE>, kLdltBlock, smem));
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(B.ninst, (int64_t)h->num_sms * std::max(per_sm, 1)));
+    const int64_t yrows = (int64_t)grid * P.N;
+    if (L->bY_rows < yrows) { L->bY.alloc((size_t)yrows + 8); L->bY_rows = yrows; }
+    B.Y = L->bY.p;
+    ldlt_batch_kernel<MODE><<<grid, kLdltBlock, smem, h->stream>>>(P, B);
+    h->launches += 1;
+    FPSB_CUDA(cudaGetLastError());
+}
+
+// kind 0: refactor every instance and solve (the factors stay in the factor store), 1: least squares with the factors of
+// the last kind-0 call.  Device pointers; factorized == NULL: the status is left in L->bok only.
+static void ldlt_batch(Handle *h, int kind, int64_t ninst, const double *jvals, const double *delta, const double *rhs1,
+                       const double *rhs2, double *p1, double *q1, double *p2, double *q2, int *factorized) {
+    LdltPlan *L = h->ldlt;
+    if (kind == 0) {
+        L->bninst = -1;
+        // grown, never shrunk; the old contents are not kept (this call refactors every instance)
+        if (L->bstore_inst < ninst) {
+            L->bstore.release(); L->bstore_inst = 0;
+            L->bstore.alloc((size_t)ninst * (size_t)L->bstride + 8);
+            L->bstore_inst = ninst;
+        }
+        if (L->bok_inst < ninst) {
+            L->bok.release(); L->bok_inst = 0;
+            L->bok.alloc((size_t)ninst + 8);
+            L->bok_inst = ninst;
+        }
+    }
+    if (!factorized) factorized = L->bok.p;
+    BatchDev B{};
+    B.sn = L->bsn.p; B.step = L->bstep.p; B.nstep = L->nbstep; B.nleaf = L->S.nleaf;
+    B.ninst = ninst; B.stride = L->bstride; B.psize = L->S.panel_size;
+    B.aslot = L->aslot.p; B.aptr = L->aptr.p; B.asrc = L->asrc.p; B.naslot = L->naslot; B.nnzj = h->nnzj;
+    B.pinv = L->pinv.p;
+    B.store = L->bstore.p; B.ok = L->bok.p;
+    B.jvals = jvals; B.delta = delta; B.rhs1 = rhs1; B.rhs2 = rhs2;
+    B.p1 = p1; B.q1 = q1; B.p2 = p2; B.q2 = q2; B.factorized = factorized;
+    B.kind = kind;
+    const int mode = ldlt_mode();
+    if (mode == 0) launch_batch<0>(h, L->dev, B);
+    else if (mode == 2) launch_batch<2>(h, L->dev, B);
+    else launch_batch<1>(h, L->dev, B);
+    if (kind == 0) L->bninst = ninst;
 }
 
 }  // namespace fpsb
@@ -1370,6 +1628,78 @@ int fpsb_ldlt_solve_two_mixed(fpsb_handle h, double delta, const double *rhs1, c
 int fpsb_ldlt_solve_two_least_squares(fpsb_handle h, const double *rhs1, const double *rhs2, double *p1,
                                       double *q1, double *p2, double *q2, int loc, int *factorized) {
     return ldlt_solve_api(h, 1, false, 0.0, rhs1, rhs2, p1, q1, p2, q2, loc, factorized);
+}
+
+static int ldlt_batch_api(fpsb_handle hh, int kind, int64_t ninst, const double *jvals, const double *delta,
+                          const double *rhs1, const double *rhs2, double *p1, double *q1, double *p2, double *q2,
+                          int *factorized, int loc) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQ(h && h->ldlt, FPSB_ESTATE, "fpsb_ldlt_analyze has not been called");
+    REQ(ninst >= 0, FPSB_EINVAL, "negative ninst");
+    REQ(loc == FPSB_HOST || loc == FPSB_DEVICE, FPSB_EINVAL, "loc must be FPSB_HOST or FPSB_DEVICE");
+    if (ninst == 0) return FPSB_OK;
+    REQ(rhs1 && rhs2 && p1 && q1 && p2 && q2 && factorized && (kind == 1 || (jvals && delta)), FPSB_EINVAL, "NULL argument");
+    REQ(kind == 0 || h->ldlt->bninst == ninst, FPSB_ESTATE,
+        "no batched factorisation of this many instances (call fpsb_ldlt_batch_solve_two_mixed first)");
+    TRY_
+    FPSB_CUDA(cudaSetDevice(h->device));
+    const size_t n = (size_t)h->nvar, m = (size_t)h->ncon, ni = (size_t)ninst, nz = (size_t)h->nnzj;
+    const size_t n2 = kind == 0 ? m : n;
+    if (loc == FPSB_DEVICE) {
+        caller_order_in(h);      // the caller's kernels wrote the inputs on its own stream
+        ldlt_batch(h, kind, ninst, jvals, delta, rhs1, rhs2, p1, q1, p2, q2, factorized);
+        caller_order_out(h);
+        return FPSB_OK;
+    }
+    // host buffers: staged through the handle's pinned area and device staging buffers (grown, never shrunk)
+    const size_t nin = (kind == 0 ? ni * nz + ni : 0) + ni * n + ni * n2;
+    const size_t nout = ni * 2 * (n + m);
+    const size_t nfac = (ni + 1) / 2;           // the int status after the doubles
+    if (h->stage_in.n < nin + 8) h->stage_in.alloc(nin + 8);
+    if (h->stage_out.n < nout + 8) h->stage_out.alloc(nout + 8);
+    const size_t need = nin + nout + nfac + 8;
+    if (h->pin_count < need) {
+        if (h->pin) cudaFreeHost(h->pin);
+        h->pin = nullptr; h->pin_count = 0;
+        FPSB_CUDA(cudaMallocHost((void **)&h->pin, need * sizeof(double)));
+        h->pin_count = need;
+    }
+    double *pin = h->pin, *din = h->stage_in.p, *dout = h->stage_out.p;
+    size_t off = 0;
+    const double *dj = nullptr, *dd = nullptr;
+    if (kind == 0) {
+        memcpy(pin, jvals, ni * nz * sizeof(double)); dj = din; off = ni * nz;
+        memcpy(pin + off, delta, ni * sizeof(double)); dd = din + off; off += ni;
+    }
+    memcpy(pin + off, rhs1, ni * n * sizeof(double));
+    const double *d1 = din + off; off += ni * n;
+    memcpy(pin + off, rhs2, ni * n2 * sizeof(double));
+    const double *d2 = din + off;
+    FPSB_CUDA(cudaMemcpyAsync(din, pin, nin * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    double *o1 = dout, *o2 = o1 + ni * n, *o3 = o2 + ni * m, *o4 = o3 + ni * n;
+    ldlt_batch(h, kind, ninst, dj, dd, d1, d2, o1, o2, o3, o4, nullptr);
+    double *res = pin + nin;
+    int *fres = reinterpret_cast<int *>(res + nout);
+    FPSB_CUDA(cudaMemcpyAsync(res, dout, nout * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    FPSB_CUDA(cudaMemcpyAsync(fres, h->ldlt->bok.p, ni * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    FPSB_CUDA(cudaStreamSynchronize(h->stream));
+    memcpy(p1, res, ni * n * sizeof(double));
+    memcpy(q1, res + ni * n, ni * m * sizeof(double));
+    memcpy(p2, res + ni * (n + m), ni * n * sizeof(double));
+    memcpy(q2, res + ni * (2 * n + m), ni * m * sizeof(double));
+    memcpy(factorized, fres, ni * sizeof(int));
+    return FPSB_OK;
+    CATCH_
+}
+
+int fpsb_ldlt_batch_solve_two_mixed(fpsb_handle h, int64_t ninst, const double *jvals, const double *delta,
+                                    const double *rhs1, const double *rhs2, double *p1, double *q1, double *p2,
+                                    double *q2, int *factorized, int loc) {
+    return ldlt_batch_api(h, 0, ninst, jvals, delta, rhs1, rhs2, p1, q1, p2, q2, factorized, loc);
+}
+int fpsb_ldlt_batch_solve_two_least_squares(fpsb_handle h, int64_t ninst, const double *rhs1, const double *rhs2,
+                                            double *p1, double *q1, double *p2, double *q2, int *factorized, int loc) {
+    return ldlt_batch_api(h, 1, ninst, nullptr, nullptr, rhs1, rhs2, p1, q1, p2, q2, factorized, loc);
 }
 
 }  // extern "C"

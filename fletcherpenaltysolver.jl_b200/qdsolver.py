@@ -245,6 +245,53 @@ class B200Handle:
         return self._two(_lib.lib().fpsb_ldlt_solve_two_least_squares,
                          "fpsb_ldlt_solve_two_least_squares", (), rhs1, rhs2, False)
 
+    # -- batched LDLt path: many instances of this handle's pattern in one call ------------------
+    def _batch(self, fn, name, pre, rhs1, rhs2, n2):
+        host = isinstance(rhs1, np.ndarray)
+        if host:
+            rhs1, rhs2 = _f64(rhs1), _f64(rhs2)
+        else:
+            import torch
+            rhs1, rhs2 = rhs1.to(torch.float64).contiguous(), rhs2.to(torch.float64).contiguous()
+        n, m = self.nvar, self.ncon
+        ninst = int(rhs1.shape[0])
+        if tuple(rhs1.shape) != (ninst, n) or tuple(rhs2.shape) != (ninst, n2):
+            raise ValueError(f"{name}: rhs1 must be (ninst, {n}) and rhs2 (ninst, {n2})")
+        p1, q1, p2, q2 = self._outs(rhs1, [(ninst, n), (ninst, m), (ninst, n), (ninst, m)])
+        if host:
+            fac = np.zeros(ninst, dtype=np.int32)
+        else:
+            import torch
+            fac = torch.zeros(ninst, dtype=torch.int32, device=rhs1.device)
+        a1, loc = self._arg(rhs1)
+        ptrs = [self._arg(a)[0] for a in (*pre, rhs2, p1, q1, p2, q2, fac)]
+        check(fn(self.h, C.c_int64(ninst), *ptrs[:len(pre)], a1, *ptrs[len(pre):], C.c_int(loc)), name)
+        return p1, q1, p2, q2, (fac.astype(bool) if host else fac.bool())
+
+    def ldlt_batch_solve_two_mixed(self, delta, jvals, rhs1, rhs2):
+        """Refactor + solve of `ninst` instances of this handle's pattern (fpsb_ldlt_batch_solve_two_mixed).
+        jvals (ninst, nnzj), rhs1 (ninst, nvar), rhs2 (ninst, ncon): numpy arrays, or CUDA tensors (device path);
+        delta: a scalar or one value per instance.  Returns p1, q1, p2, q2 as (ninst, .) arrays and `factorized`
+        (bool, per instance).  The factors stay on the device for ldlt_batch_solve_two_least_squares."""
+        ninst = int(rhs1.shape[0])
+        if isinstance(rhs1, np.ndarray):
+            jvals = _f64(jvals)
+            d = _f64(np.broadcast_to(np.asarray(delta, dtype=np.float64), (ninst,)))
+        else:
+            import torch
+            jvals = torch.as_tensor(jvals, dtype=torch.float64, device=rhs1.device).contiguous()
+            d = torch.as_tensor(delta, dtype=torch.float64, device=rhs1.device).expand(ninst).contiguous()
+        if tuple(jvals.shape) != (ninst, self.nnzj):
+            raise ValueError(f"ldlt_batch_solve_two_mixed: jvals must be (ninst, {self.nnzj})")
+        return self._batch(_lib.lib().fpsb_ldlt_batch_solve_two_mixed, "fpsb_ldlt_batch_solve_two_mixed",
+                           (jvals, d), rhs1, rhs2, self.ncon)
+
+    def ldlt_batch_solve_two_least_squares(self, rhs1, rhs2):
+        """Least-squares solves of the instances of the last ldlt_batch_solve_two_mixed call (same ninst) with their
+        stored factors; rhs1, rhs2 (ninst, nvar)."""
+        return self._batch(_lib.lib().fpsb_ldlt_batch_solve_two_least_squares,
+                           "fpsb_ldlt_batch_solve_two_least_squares", (), rhs1, rhs2, self.nvar)
+
 
 # --------------------------------------------------------------------------------------------------
 # plugin surface
@@ -412,6 +459,45 @@ def solve_two_extras(fpnlp, x, rhs1, rhs2):
         qds.last_stats = st
         return u1, u2
     raise TypeError(f"solve_two_extras: no method for {type(qds).__name__}")
+
+
+def solve_two_mixed_batch(fpnlp, X, rhs1, rhs2, delta=None):
+    """solve_two_mixed at every row of X in one batched call (LDLtSolver only): instance i is
+    solve_two_mixed(fpnlp, X[i], rhs1[i], rhs2[i]) with delta[i] (default fpnlp.delta for all), the Jacobian values
+    evaluated at X[i] (jac_coord / jac_nln_coord, as solve_two_mixed does).  Returns p1, q1, p2, q2 as (ninst, .)
+    arrays; warns once per instance whose factorisation failed.  The factors are kept for
+    solve_two_least_squares_batch."""
+    qds = fpnlp.qdsolver
+    if not isinstance(qds, LDLtSolver):
+        raise TypeError(f"solve_two_mixed_batch: no method for {type(qds).__name__}")
+    H = qds.handle
+    X = np.asarray(X, dtype=np.float64)
+    J = np.empty((X.shape[0], H.nnzj))
+    for i, x in enumerate(X):
+        J[i] = _jac_values(fpnlp, x)
+    if not isinstance(rhs1, np.ndarray):
+        import torch
+        J = torch.as_tensor(J, device=rhs1.device)
+    p1, q1, p2, q2, ok = H.ldlt_batch_solve_two_mixed(float(fpnlp.delta) if delta is None else delta, J, rhs1, rhs2)
+    _warn_failed(ok)
+    return p1, q1, p2, q2
+
+
+def solve_two_least_squares_batch(fpnlp, X, rhs1, rhs2):
+    """solve_two_least_squares for the instances of the last solve_two_mixed_batch call (same number of rows): the
+    factorisations of that call are trusted, as the single-instance function trusts the last solve_two_mixed."""
+    qds = fpnlp.qdsolver
+    if not isinstance(qds, LDLtSolver):
+        raise TypeError(f"solve_two_least_squares_batch: no method for {type(qds).__name__}")
+    p1, q1, p2, q2, ok = qds.handle.ldlt_batch_solve_two_least_squares(rhs1, rhs2)
+    _warn_failed(ok)
+    return p1, q1, p2, q2
+
+
+def _warn_failed(ok):
+    failed = int((~ok).sum()) if isinstance(ok, np.ndarray) else int((~ok).sum().item())
+    for _ in range(failed):
+        warnings.warn("_solve_ldlt_factorization: failed _factorization")
 
 
 def batch_solve_two(A, delta, rhs1, rhs2, kind="mixed", opts=None, device=0):

@@ -228,6 +228,25 @@ int fpsb_ldlt_solve_two_least_squares(fpsb_handle h, const double *rhs1, const d
 int fpsb_ldlt_solve_two_extras(fpsb_handle h, double delta, const double *rhs1, const double *rhs2,
                                double *u1, double *u2, int loc, fpsb_krylov_stats stats[2]);
 
+/* Batched LDLt path: `ninst` instances that share this handle's Jacobian pattern and its symbolic analysis
+ * (fpsb_ldlt_analyze must have run), each with its own Jacobian values, delta and right-hand sides; one kernel launch
+ * per call, one CTA per instance at a time.  Per-entry results are those of the single-instance entries above run on
+ * each instance alone (same routines, same operation order).
+ *   jvals [ninst][nnzj] (COO order given to fpsb_create), delta [ninst],
+ *   rhs1 [ninst][nvar], rhs2 [ninst][ncon] (mixed) or [ninst][nvar] (least squares),
+ *   p1, p2 [ninst][nvar], q1, q2 [ninst][ncon], factorized [ninst] (where `loc` says, like the outputs).
+ * mixed = refactor + solve of every instance (src/solve_linear_system.jl:206-252); the factors stay on the device
+ * (ninst x (panel_nnz + nvar + ncon) doubles, grown and never shrunk) and
+ * fpsb_ldlt_batch_solve_two_least_squares (:161-204) reuses them (same ninst required, FPSB_ESTATE otherwise).
+ * An instance whose factorisation fails gets factorized[i] = 0 and its right-hand sides as outputs (:242-251).
+ * ninst == 0 is a no-op.  The single-instance factor, values and state of the handle are left alone.  With
+ * loc = FPSB_DEVICE the call is asynchronous, ordered against the caller's stream (fpsb_set_caller_stream). */
+int fpsb_ldlt_batch_solve_two_mixed(fpsb_handle h, int64_t ninst, const double *jvals, const double *delta,
+                                    const double *rhs1, const double *rhs2, double *p1, double *q1, double *p2,
+                                    double *q2, int *factorized, int loc);
+int fpsb_ldlt_batch_solve_two_least_squares(fpsb_handle h, int64_t ninst, const double *rhs1, const double *rhs2,
+                                            double *p1, double *q1, double *p2, double *q2, int *factorized, int loc);
+
 /* ---------------------------------------------------------------------------------------------
  * Throughput mode — many independent SMALL instances (BASELINE config C5): the LDLt path of
  * solve_two_mixed (kind 0, src/solve_linear_system.jl:206-252) or solve_two_least_squares (kind 1,

@@ -42,6 +42,13 @@ class LdltOpts(C.Structure):
     _fields_ = [("ldlt_tol", C.c_double), ("ldlt_r1", C.c_double), ("ldlt_r2", C.c_double)]
 
 
+class ExtrasOpts(C.Structure):
+    """fpsb_extras_opts — tolerances of the batched LDLt solve_two_extras (itmax 0 = Krylov.jl's default)."""
+    _fields_ = [("cg_atol", C.c_double), ("cg_rtol", C.c_double), ("cg_itmax", C.c_int64),
+                ("mr_atol", C.c_double), ("mr_rtol", C.c_double), ("mr_etol", C.c_double),
+                ("mr_conlim", C.c_double), ("mr_itmax", C.c_int64)]
+
+
 # every symbol include/fpsb.h declares (checked by tests/test_abi.py)
 EXPORTS = [
     "fpsb_version", "fpsb_last_error", "fpsb_device_count", "fpsb_create", "fpsb_destroy",
@@ -52,7 +59,7 @@ EXPORTS = [
     "fpsb_ldlt_analyze", "fpsb_ldlt_symbolic_sizes", "fpsb_ldlt_get_symbolic",
     "fpsb_ldlt_plan_info", "fpsb_ldlt_factorize", "fpsb_ldlt_get_factor",
     "fpsb_ldlt_solve_two_mixed", "fpsb_ldlt_solve_two_least_squares", "fpsb_ldlt_solve_two_extras",
-    "fpsb_ldlt_batch_solve_two_mixed", "fpsb_ldlt_batch_solve_two_least_squares",
+    "fpsb_ldlt_batch_solve_two_mixed", "fpsb_ldlt_batch_solve_two_least_squares", "fpsb_ldlt_batch_solve_two_extras",
     "fpsb_symbolic_create", "fpsb_symbolic_destroy", "fpsb_symbolic_sizes", "fpsb_symbolic_get",
     "fpsb_symbolic_plan_info", "fpsb_order_dissection", "fpsb_batch_solve_two",
     "fpsb_dist_unique_id", "fpsb_dist_attach", "fpsb_dist_jprod", "fpsb_dist_jtprod",

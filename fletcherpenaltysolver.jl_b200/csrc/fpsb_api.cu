@@ -174,6 +174,7 @@ int fpsb_destroy(fpsb_handle hh) {
     dist_free(h);
     fp_free(h);
     iter_free(h);
+    extras_free(h);
     ldlt_free(h);
     if (h->pin) cudaFreeHost(h->pin);
     if (h->ev0) cudaEventDestroy(h->ev0);
@@ -406,6 +407,32 @@ int fpsb_iter_solve_two_extras(fpsb_handle h, double delta, const double *rhs1, 
 int fpsb_ldlt_solve_two_extras(fpsb_handle h, double delta, const double *rhs1, const double *rhs2,
                                double *u1, double *u2, int loc, fpsb_krylov_stats stats[2]) {
     return extras(h, true, delta, rhs1, rhs2, u1, u2, loc, stats);
+}
+
+// batched LDLt solve_two_extras: host buffers go through the handle's pinned area and stage buffers (Staged); device
+// buffers are stream-ordered against the caller and the call returns without waiting for the result
+int fpsb_ldlt_batch_solve_two_extras(fpsb_handle hh, int64_t ninst, const double *jvals, const double *delta,
+                                     const double *rhs1, const double *rhs2, double *u1, double *u2,
+                                     fpsb_krylov_stats *stats, const fpsb_extras_opts *opts, int loc) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQUIRE(h, FPSB_EINVAL, "NULL handle");
+    REQUIRE(ninst >= 0, FPSB_EINVAL, "negative ninst");
+    REQUIRE(loc == FPSB_HOST || loc == FPSB_DEVICE, FPSB_EINVAL, "loc must be FPSB_HOST or FPSB_DEVICE");
+    if (ninst == 0) return FPSB_OK;
+    REQUIRE(jvals && delta && rhs1 && rhs2 && u1 && u2 && stats, FPSB_EINVAL, "NULL argument");
+    REQUIRE(!opts || (opts->cg_itmax >= 0 && opts->mr_itmax >= 0), FPSB_EINVAL, "negative itmax");
+    FPSB_TRY
+    FPSB_CUDA(cudaSetDevice(h->device));
+    const size_t n = (size_t)h->nvar, m = (size_t)h->ncon, ni = (size_t)ninst, nz = (size_t)h->nnzj;
+    const size_t sw = sizeof(fpsb_krylov_stats) / sizeof(double);     // the stats travel as doubles
+    Staged S(h, loc, ni * nz + ni + ni * n + ni * m, 2 * ni * m + 2 * ni * sw);
+    const double *dj = S.in(jvals, ni * nz), *dd = S.in(delta, ni), *d1 = S.in(rhs1, ni * n), *d2 = S.in(rhs2, ni * m);
+    double *o1 = S.out(u1, ni * m), *o2 = S.out(u2, ni * m);
+    fpsb_krylov_stats *ost = reinterpret_cast<fpsb_krylov_stats *>(S.out(reinterpret_cast<double *>(stats), 2 * ni * sw));
+    extras_batch(h, ninst, dj, dd, d1, d2, o1, o2, ost, opts);
+    S.finish(false);
+    return FPSB_OK;
+    FPSB_CATCH
 }
 
 /* ---- row-partitioned Krylov over NCCL (SURVEY 8e) ------------------------------------------------ */

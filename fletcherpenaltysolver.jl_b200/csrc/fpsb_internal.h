@@ -106,6 +106,7 @@ struct IterWs;     // defined in fpsb_krylov.cu
 struct LdltPlan;   // defined in fpsb_ldlt.cu
 struct DistCtx;    // defined in fpsb_dist.inl (row-partitioned multi-GPU runs)
 struct FpWs;       // defined in fpsb_fpnlp.cu
+struct ExtrasWs;   // defined in fpsb_extras_batch.inl
 
 struct Handle {
     int device = 0;
@@ -131,6 +132,7 @@ struct Handle {
     LdltPlan *ldlt = nullptr;
     DistCtx *dist = nullptr;
     FpWs *fp = nullptr;
+    ExtrasWs *extras = nullptr;               // batched solve_two_extras: CSR patterns + workspace (built at first use)
     fpsb_iter_opts iopts{};
     bool iopts_set = false;
     double prof_loop_ms = 0.0;          // CUDA-event time of the last Krylov loop region
@@ -157,6 +159,11 @@ void iter_solve_two_least_squares(Handle *h, double delta, const double *rhs1, c
                                   fpsb_krylov_stats *st);
 void iter_solve_two_extras(Handle *h, double delta, const double *rhs1, const double *rhs2, double *u1,
                            double *u2, fpsb_krylov_stats *st, bool ldlt_variant);
+// fpsb_extras_batch.inl: solve_two_extras of the LDLt path for ninst instances of the handle's pattern (device
+// buffers, stream-ordered on h->stream); opts == nullptr: the single-instance entry's tolerances
+void extras_batch(Handle *h, int64_t ninst, const double *jvals, const double *delta, const double *rhs1,
+                  const double *rhs2, double *u1, double *u2, fpsb_krylov_stats *stats, const fpsb_extras_opts *opts);
+void extras_free(Handle *h);
 
 // fpsb_dist.inl (row-partitioned Krylov over NCCL)
 void dist_unique_id(void *out128);

@@ -2162,26 +2162,29 @@ static SlotState make_craig(double delta, double atol, double rtol, double btol,
     S.active = 1;
     return S;
 }
-static SlotState make_minres(double lambda, double atol, double rtol, double etol, double conlim,
-                             int64_t itmax, int64_t n_op) {
+// make_minres / make_cgls also run on the device: the batched extras kernel (fpsb_extras_batch.inl) sets up every
+// instance's state from its own delta with them
+static __host__ __device__ SlotState make_minres(double lambda, double atol, double rtol, double etol, double conlim,
+                                                 int64_t itmax, int64_t n_op) {
     SlotState S;
     memset(&S, 0, sizeof(S));
     S.algo = ALGO_MINRES;
     S.lambda = lambda; S.atol = atol; S.rtol = rtol; S.etol = etol;
     S.ctol = conlim > 0 ? 1.0 / conlim : 0.0;
     int64_t im = itmax == 0 ? 2 * n_op : itmax;
-    S.itmax = (int)std::min<int64_t>(im, 2000000000);
+    S.itmax = (int)(im < 2000000000 ? im : 2000000000);
     S.active = 1;
     S.mscale = 1.0;
     return S;
 }
-static SlotState make_cgls(double lambda, double atol, double rtol, int64_t itmax, int64_t m_op, int64_t n_op) {
+static __host__ __device__ SlotState make_cgls(double lambda, double atol, double rtol, int64_t itmax, int64_t m_op,
+                                               int64_t n_op) {
     SlotState S;
     memset(&S, 0, sizeof(S));
     S.algo = ALGO_CGLS;
     S.lambda = lambda; S.atol = atol; S.rtol = rtol;
     int64_t im = itmax == 0 ? m_op + n_op : itmax;
-    S.itmax = (int)std::min<int64_t>(im, 2000000000);
+    S.itmax = (int)(im < 2000000000 ? im : 2000000000);
     S.active = 1;
     S.mscale = 1.0;
     return S;
@@ -2195,7 +2198,7 @@ static SlotState make_none() {
     return S;
 }
 
-static void stats_from(const SlotState &S, fpsb_krylov_stats &o) {
+static __host__ __device__ void stats_from(const SlotState &S, fpsb_krylov_stats &o) {
     o.niter = S.iter; o.solved = S.solved; o.inconsistent = S.inconsistent; o.status = S.status;
     o.pad_ = 0;
     o.rnorm = S.rNorm; o.arnorm = S.ArNorm; o.anorm = S.Anorm; o.acond = S.Acond; o.xnorm = S.xNorm;
@@ -2659,6 +2662,7 @@ void iter_solve_two_extras(Handle *h, double delta, const double *rhs1, const do
     }
 }
 
+#include "fpsb_extras_batch.inl"
 
 #include "fpsb_dist.inl"
 

@@ -18,7 +18,7 @@ import warnings
 import numpy as np
 
 from . import _lib
-from ._lib import FPSB_DEVICE, FPSB_HOST, IterOpts, KrylovStats, LdltOpts, check
+from ._lib import FPSB_DEVICE, FPSB_HOST, ExtrasOpts, IterOpts, KrylovStats, LdltOpts, check
 
 SQRT_EPS = float(np.sqrt(np.finfo(np.float64).eps))
 
@@ -292,6 +292,63 @@ class B200Handle:
         return self._batch(_lib.lib().fpsb_ldlt_batch_solve_two_least_squares,
                            "fpsb_ldlt_batch_solve_two_least_squares", (), rhs1, rhs2, self.nvar)
 
+    def ldlt_batch_solve_two_extras(self, delta, jvals, rhs1, rhs2, opts=None):
+        """solve_two_extras of the LDLt path for `ninst` instances of this handle's pattern
+        (fpsb_ldlt_batch_solve_two_extras): u1 = cgls(A', rhs1, lambda = tau), u2 = minres(A A', rhs2, lambda = tau),
+        tau = max(delta, 1e-14), with each instance's own Jacobian values.  jvals (ninst, nnzj), rhs1 (ninst, nvar),
+        rhs2 (ninst, ncon): numpy arrays, or CUDA tensors (device path); delta: a scalar or one value per instance;
+        opts: an ExtrasOpts (None: the tolerances of ldlt_solve_two_extras).  Needs neither ldlt_analyze nor
+        set_jac_values and changes neither.  Returns u1, u2 as (ninst, ncon) arrays and the stats as a dict of
+        (ninst, 2) arrays (column 0 CGLS, column 1 MINRES) keyed like KrylovStats.as_dict()."""
+        host = isinstance(rhs1, np.ndarray)
+        n, m, name = self.nvar, self.ncon, "ldlt_batch_solve_two_extras"
+        if host:
+            rhs1, rhs2, jvals = _f64(rhs1), _f64(rhs2), _f64(jvals)
+            d = np.asarray(delta, dtype=np.float64)
+        else:
+            import torch
+            dev = rhs1.device
+            rhs1, rhs2 = rhs1.to(torch.float64).contiguous(), rhs2.to(torch.float64).contiguous()
+            jvals = torch.as_tensor(jvals, dtype=torch.float64, device=dev).contiguous()
+            d = torch.as_tensor(delta, dtype=torch.float64, device=dev)
+        ninst = int(rhs1.shape[0]) if rhs1.ndim == 2 else -1
+        if (ninst < 0 or tuple(rhs1.shape) != (ninst, n) or tuple(rhs2.shape) != (ninst, m)
+                or tuple(jvals.shape) != (ninst, self.nnzj)):
+            raise ValueError(f"{name}: jvals must be (ninst, {self.nnzj}), rhs1 (ninst, {n}) and rhs2 (ninst, {m})")
+        if d.ndim == 0:
+            d = np.full(ninst, float(d)) if host else d.expand(ninst).contiguous()
+        elif tuple(d.shape) != (ninst,):
+            raise ValueError(f"{name}: delta must be a scalar or have one value per instance")
+        else:
+            d = _f64(d) if host else d.contiguous()
+        u1, u2 = self._outs(rhs1, [(ninst, m), (ninst, m)])
+        # fpsb_krylov_stats [ninst][2] is 8 doubles per entry
+        if host:
+            st = np.zeros((ninst, 2, 8))
+        else:
+            import torch
+            st = torch.zeros((ninst, 2, 8), dtype=torch.float64, device=rhs1.device)
+        a1, loc = self._arg(rhs1)
+        ptrs = [self._arg(a)[0] for a in (jvals, d, rhs2, u1, u2, st)]
+        check(_lib.lib().fpsb_ldlt_batch_solve_two_extras(
+            self.h, C.c_int64(ninst), ptrs[0], ptrs[1], a1, *ptrs[2:],
+            C.byref(opts) if opts is not None else None, C.c_int(loc)), "fpsb_ldlt_batch_solve_two_extras")
+        return u1, u2, _stats_arrays(st, host)
+
+
+def _stats_arrays(st, host):
+    """(ninst, 2, 8) float64 view of fpsb_krylov_stats [ninst][2] -> dict of (ninst, 2) arrays (KrylovStats layout:
+    niter int64 | solved, inconsistent, status, pad int32 | rnorm, arnorm, anorm, acond, xnorm)."""
+    if host:
+        i64, i32, cp = st.view(np.int64), st.view(np.int32), np.copy
+    else:
+        import torch
+        i64, i32, cp = st.view(torch.int64), st.view(torch.int32), torch.clone
+    out = dict(niter=cp(i64[..., 0]), solved=i32[..., 2] != 0, inconsistent=i32[..., 3] != 0, status=cp(i32[..., 4]))
+    for k, name in enumerate(("rnorm", "arnorm", "anorm", "acond", "xnorm")):
+        out[name] = cp(st[..., 3 + k])
+    return out
+
 
 # --------------------------------------------------------------------------------------------------
 # plugin surface
@@ -375,6 +432,7 @@ class LDLtSolver(QDSolver):
         self.handle.ldlt_analyze(P, 0, o)
         self.factorized = False
         self.last_stats = None
+        self.last_batch_stats = None
 
 
 qdsolver_correspondence = {"iterative": IterativeSolver, "ldlt": LDLtSolver}
@@ -492,6 +550,28 @@ def solve_two_least_squares_batch(fpnlp, X, rhs1, rhs2):
     p1, q1, p2, q2, ok = qds.handle.ldlt_batch_solve_two_least_squares(rhs1, rhs2)
     _warn_failed(ok)
     return p1, q1, p2, q2
+
+
+def solve_two_extras_batch(fpnlp, X, rhs1, rhs2, delta=None):
+    """solve_two_extras at every row of X in one batched call (LDLtSolver only): instance i is
+    solve_two_extras(fpnlp, X[i], rhs1[i], rhs2[i]) with delta[i] (default fpnlp.delta for all), the Jacobian values
+    evaluated at X[i] (jac_coord / jac_nln_coord, as solve_two_extras does).  rhs1 (ninst, nvar), rhs2 (ninst, npen).
+    Returns u1, u2 as (ninst, npen) arrays; the per-instance Krylov stats go to qdsolver.last_batch_stats.  Like the
+    single LDLt solve_two_extras it does not warn.  Leaves the factors of solve_two_mixed_batch alone."""
+    qds = fpnlp.qdsolver
+    if not isinstance(qds, LDLtSolver):
+        raise TypeError(f"solve_two_extras_batch: no method for {type(qds).__name__}")
+    H = qds.handle
+    X = np.asarray(X, dtype=np.float64)
+    J = np.empty((X.shape[0], H.nnzj))
+    for i, x in enumerate(X):
+        J[i] = _jac_values(fpnlp, x)
+    if not isinstance(rhs1, np.ndarray):
+        import torch
+        J = torch.as_tensor(J, device=rhs1.device)
+    u1, u2, st = H.ldlt_batch_solve_two_extras(float(fpnlp.delta) if delta is None else delta, J, rhs1, rhs2)
+    qds.last_batch_stats = st
+    return u1, u2
 
 
 def _warn_failed(ok):

@@ -247,6 +247,30 @@ int fpsb_ldlt_batch_solve_two_mixed(fpsb_handle h, int64_t ninst, const double *
 int fpsb_ldlt_batch_solve_two_least_squares(fpsb_handle h, int64_t ninst, const double *rhs1, const double *rhs2,
                                             double *p1, double *q1, double *p2, double *q2, int *factorized, int loc);
 
+/* Tolerances of fpsb_ldlt_batch_solve_two_extras; NULL = what the reference's LDLt call uses, i.e. exactly what
+ * fpsb_ldlt_solve_two_extras runs (Krylov.jl defaults: cgls atol = rtol = sqrt(eps), itmax = nvar + ncon; minres
+ * atol = rtol = sqrt(eps)/100, etol = sqrt(eps), conlim = 1/sqrt(eps), itmax = 2 ncon).  itmax == 0 means that
+ * default; a negative itmax is FPSB_EINVAL. */
+typedef struct {
+    double cg_atol, cg_rtol; int64_t cg_itmax;
+    double mr_atol, mr_rtol, mr_etol, mr_conlim; int64_t mr_itmax;
+} fpsb_extras_opts;
+/* Batched solve_two_extras [LDLt]  src/solve_linear_system.jl:142-159: for each of `ninst` instances of this handle's
+ * Jacobian pattern, u1 = cgls(A', rhs1, lambda = tau) and u2 = minres(A A', rhs2, lambda = tau), tau = max(delta, 1e-14),
+ * with the instance's own Jacobian values.  One kernel launch per call: every (instance, method) pair runs inside one
+ * CTA, with fixed-order reductions, so results are bitwise reproducible and do not depend on the batch (size, position)
+ * or on `loc`; they agree with fpsb_ldlt_solve_two_extras on the same instance to the Krylov tolerances (its reductions
+ * span many CTAs and round differently).
+ *   jvals [ninst][nnzj] (COO order given to fpsb_create), delta [ninst], rhs1 [ninst][nvar], rhs2 [ninst][ncon],
+ *   u1, u2 [ninst][ncon], stats [ninst][2] (CGLS, MINRES; where `loc` says, like the outputs).
+ * Runs on any handle: it needs neither fpsb_ldlt_analyze nor fpsb_set_jac_values, and leaves the handle's
+ * single-instance values, Krylov workspaces and the factors of fpsb_ldlt_batch_solve_two_mixed alone (mixed -> least
+ * squares -> extras is the Val(1) hprod order).  ninst == 0 is a no-op.  With loc = FPSB_DEVICE the call is
+ * asynchronous, ordered against the caller's stream (fpsb_set_caller_stream). */
+int fpsb_ldlt_batch_solve_two_extras(fpsb_handle h, int64_t ninst, const double *jvals, const double *delta,
+                                     const double *rhs1, const double *rhs2, double *u1, double *u2,
+                                     fpsb_krylov_stats *stats, const fpsb_extras_opts *opts, int loc);
+
 /* ---------------------------------------------------------------------------------------------
  * Throughput mode — many independent SMALL instances (BASELINE config C5): the LDLt path of
  * solve_two_mixed (kind 0, src/solve_linear_system.jl:206-252) or solve_two_least_squares (kind 1,

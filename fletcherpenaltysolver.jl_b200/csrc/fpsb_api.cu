@@ -337,6 +337,12 @@ int fpsb_iter_last_profile(fpsb_handle hh, double *loop_ms, int64_t *step_launch
     if (step_launches) *step_launches = h->prof_step_launches;
     return FPSB_OK;
 }
+int fpsb_iter_loop_info(fpsb_handle hh, int64_t out[8]) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQUIRE(h && out, FPSB_EINVAL, "fpsb_iter_loop_info: NULL argument");
+    for (int i = 0; i < 8; ++i) out[i] = h->loop_info[i];
+    return FPSB_OK;
+}
 
 // Pipelined throughput mode (several handles of one process driven by their own host threads): one solve COMPUTES at
 // a time per device.  The H2D copies of a waiting handle are already enqueued on its stream and the D2H of a finished

@@ -137,6 +137,9 @@ struct Handle {
     bool iopts_set = false;
     double prof_loop_ms = 0.0;          // CUDA-event time of the last Krylov loop region
     int64_t prof_step_launches = 0;     // fused SpMM step kernels launched in that region
+    // geometry the persistent loop of the last Krylov solve ran with (fpsb_iter_loop_info): persistent, early,
+    // nstage, grid, stage_bytes, inflight, nspec, chunk iterations; all zero when that solve took the step path
+    int64_t loop_info[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 };
 
 // api.cu: stream ordering against the caller of FPSB_DEVICE entries

@@ -2213,6 +2213,7 @@ struct Engine {
     unsigned long long pt_sig = 0;
     int pt_par = 0;
     Engine(Handle *hh) : h(hh), W(hh->iter) {
+        memset(h->loop_info, 0, sizeof(h->loop_info));      // run_loop fills it in if this solve runs the persistent loop
         memset(&base_m, 0, sizeof(base_m));
         memset(&base_n, 0, sizeof(base_n));
         fill_csr(base_m, h->A);
@@ -2366,6 +2367,11 @@ struct Engine {
         L.parts = W->loop_parts.p;
         L.gbar = W->gbar.p;
         L.done_flag = W->done.p;
+        {
+            const int64_t info[8] = {1, L.early, nstage, grid, stage_bytes, std::max(L.op[0].inflight, L.op[1].inflight),
+                                     L.nspec, chunk_it};
+            memcpy(h->loop_info, info, sizeof(info));
+        }
         const size_t smem = (size_t)nstage * (size_t)stage_bytes;
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(kStepThreads);
@@ -2455,6 +2461,7 @@ static bool degenerate_two(Handle *h, int kind, double delta, const double *rhs1
                            double *p2, double *q2, fpsb_krylov_stats *st) {
     const int64_t n = h->nvar, m = h->ncon;
     if (n > 0 && m > 0) return false;
+    memset(h->loop_info, 0, sizeof(h->loop_info));
     auto fill = [&](int64_t cnt, double *dst, const double *src, double c) {
         if (cnt > 0) { fill_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, h->stream>>>((int)cnt, dst, src, c); h->launches += 1; }
     };
@@ -2611,6 +2618,7 @@ void iter_solve_two_extras(Handle *h, double delta, const double *rhs1, const do
     if (h->nvar == 0 || h->ncon == 0) {
         // (A A' + tau I) u = rhs with no variables: u1 = 0 (A rhs1 is empty), u2 = rhs2 / tau ; no constraints: nothing
         const double tau = std::max(delta, 1e-14);
+        memset(h->loop_info, 0, sizeof(h->loop_info));
         if (h->ncon > 0) {
             fill_kernel<<<(unsigned)((h->ncon + 255) / 256), 256, 0, h->stream>>>((int)h->ncon, u1, nullptr, 0.0);
             fill_kernel<<<(unsigned)((h->ncon + 255) / 256), 256, 0, h->stream>>>((int)h->ncon, u2, rhs2, 1.0 / tau);

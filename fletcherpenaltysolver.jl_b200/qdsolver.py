@@ -174,6 +174,13 @@ class B200Handle:
         check(_lib.lib().fpsb_iter_last_profile(self.h, C.byref(ms), C.byref(nl)), "fpsb_iter_last_profile")
         return ms.value, nl.value
 
+    def loop_info(self):
+        """Persistent-loop geometry of the last iter_solve_two_* call (fpsb_iter_loop_info)."""
+        out = (C.c_int64 * 8)()
+        check(_lib.lib().fpsb_iter_loop_info(self.h, out), "fpsb_iter_loop_info")
+        keys = ("persistent", "early", "nstage", "grid", "stage_bytes", "inflight", "nspec", "chunk")
+        return {k: int(v) for k, v in zip(keys, out)}
+
     def iter_solve_two_mixed(self, delta, rhs1, rhs2, out=None):
         return self._two(_lib.lib().fpsb_iter_solve_two_mixed, "fpsb_iter_solve_two_mixed",
                          (C.c_double(delta),), rhs1, rhs2, True, out)

@@ -159,6 +159,11 @@ int fpsb_iter_solve_two_least_squares(fpsb_handle h, double delta, const double 
 /* CUDA-event time (ms) of the Krylov loop region of the last solve_two_mixed/_least_squares call
  * on this handle and the number of fused SpMM step kernels launched in it (bench.py roofline). */
 int fpsb_iter_last_profile(fpsb_handle h, double *loop_ms, int64_t *step_launches);
+/* Geometry of the persistent Krylov loop kernel in the last iter_solve_two_* call on this handle, as launched:
+ * out = {persistent kernel used (0/1), early row sums (0/1), ring stages, grid (CTAs), bytes per ring stage, tiles a
+ * step-kernel producer may have in flight, tiles requested before a phase is decided, iterations per launch}.
+ * All zero when that solve ran one launch per half iteration.  Host only: touches nothing on the device. */
+int fpsb_iter_loop_info(fpsb_handle h, int64_t out[8]);
 /* solve_two_extras [Iterative]  src/solve_linear_system.jl:45-77
  *   u1 = LSQR(A', rhs1, lambda = sqrt(tau)); u2 = MINRES(A A', rhs2, lambda = tau), tau = max(delta,1e-14) */
 int fpsb_iter_solve_two_extras(fpsb_handle h, double delta, const double *rhs1, const double *rhs2,

@@ -10,14 +10,14 @@ from .qdsolver import (B200Handle, IterativeSolver, LDLtSolver, QDSolver, batch_
                        solve_two_extras, solve_two_extras_batch, solve_two_least_squares, solve_two_least_squares_batch,
                        solve_two_mixed, solve_two_mixed_batch)
 from .fletcher_nlp import FletcherPenaltyNLP
-from .device_nlp import DeviceCurvedQP, DeviceFletcherPenaltyNLP, DeviceSparseQP
+from .device_nlp import BatchFletcherPenaltyNLP, DeviceCurvedQP, DeviceFletcherPenaltyNLP, DeviceSparseQP
 from .fps_solve import AlgoData, FPSSSolver, GenericExecutionStats, GNSolver, fps_solve, solve, trunk
 from . import models
 
 __all__ = ["B200Handle", "IterativeSolver", "LDLtSolver", "QDSolver", "qdsolver_correspondence",
            "solve_two_extras", "solve_two_extras_batch", "solve_two_least_squares", "solve_two_mixed", "solve_two_least_squares_batch",
            "solve_two_mixed_batch", "FletcherPenaltyNLP",
-           "DeviceFletcherPenaltyNLP", "DeviceSparseQP", "DeviceCurvedQP", "fps_solve", "FPSSSolver", "AlgoData", "GNSolver",
+           "DeviceFletcherPenaltyNLP", "BatchFletcherPenaltyNLP", "DeviceSparseQP", "DeviceCurvedQP", "fps_solve", "FPSSSolver", "AlgoData", "GNSolver",
            "GenericExecutionStats", "solve", "trunk",
            "models", "batch_solve_two", "FPSB_HOST", "FPSB_DEVICE", "FpsbError", "IterOpts", "KrylovStats", "LdltOpts",
            "ExtrasOpts"]

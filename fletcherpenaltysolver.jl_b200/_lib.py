@@ -66,6 +66,9 @@ EXPORTS = [
     "fpsb_dist_solve_two_mixed", "fpsb_dist_solve_two_least_squares", "fpsb_dist_solve_two_extras", "fpsb_dist_profile", "fpsb_dist_last_profile",
     "fpsb_dist_peer_blob_bytes", "fpsb_dist_peer_export", "fpsb_dist_peer_attach", "fpsb_dist_peer_active",
     "fpsb_fp_ys_gs", "fpsb_fp_hash", "fpsb_fp_obj", "fpsb_fp_grad", "fpsb_fp_ptv", "fpsb_fp_hprod2", "fpsb_fp_hprod1", "fpsb_trcg_init", "fpsb_trcg_step",
+    "fpsb_fp_batch_ys_gs", "fpsb_fp_batch_hash", "fpsb_fp_batch_obj", "fpsb_fp_batch_grad", "fpsb_fp_batch_ptv",
+    "fpsb_fp_batch_hprod2", "fpsb_fp_batch_hprod1", "fpsb_batch_jprod", "fpsb_batch_jtprod", "fpsb_trcg_batch_init",
+    "fpsb_trcg_batch_step",
 ]
 
 _lib = None

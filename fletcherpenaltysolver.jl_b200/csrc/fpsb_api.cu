@@ -677,4 +677,115 @@ int fpsb_fp_hash(fpsb_handle hh, const double *x, uint64_t *key) {
     FPSB_CATCH
 }
 
+/* ---- the same glue for many instances of one model; all arguments are DEVICE pointers, instance-major ---- */
+#define FPB_BEGIN(name)                                                       \
+    Handle *h = reinterpret_cast<Handle *>(hh);                               \
+    REQUIRE(h, FPSB_EINVAL, name ": NULL handle");                            \
+    REQUIRE(ninst >= 0, FPSB_EINVAL, name ": negative ninst");                \
+    if (ninst == 0) return FPSB_OK;
+#define FPB_RUN(call)                                                         \
+    FPSB_TRY                                                                  \
+    FPSB_CUDA(cudaSetDevice(h->device));                                      \
+    caller_order_in(h);                                                       \
+    call;                                                                     \
+    caller_order_out(h);                                                      \
+    return FPSB_OK;                                                           \
+    FPSB_CATCH
+
+int fpsb_fp_batch_ys_gs(fpsb_handle hh, int64_t ninst, const double *sigma, const double *p1, const double *q1,
+                        const double *p2, const double *q2, double *gs, double *ys, double *v, double *w) {
+    FPB_BEGIN("fpsb_fp_batch_ys_gs")
+    REQUIRE(sigma && p1 && q1 && p2 && q2 && gs && ys && v && w, FPSB_EINVAL, "fpsb_fp_batch_ys_gs: NULL argument");
+    FPB_RUN(fpb_ys_gs(h, ninst, sigma, p1, q1, p2, q2, gs, ys, v, w))
+}
+int fpsb_fp_batch_hash(fpsb_handle hh, int64_t ninst, const double *x, uint64_t *keys) {
+    FPB_BEGIN("fpsb_fp_batch_hash")
+    REQUIRE(keys && (x || h->nvar == 0), FPSB_EINVAL, "fpsb_fp_batch_hash: NULL argument");
+    FPB_RUN(fpb_hash(h, ninst, x, keys))
+}
+int fpsb_fp_batch_obj(fpsb_handle hh, int64_t ninst, const double *fx, const double *rho, const double *eta, const double *c,
+                      const double *ys, const double *x, const double *xk, double *phi) {
+    FPB_BEGIN("fpsb_fp_batch_obj")
+    REQUIRE(fx && phi && ((c && ys) || h->ncon == 0), FPSB_EINVAL, "fpsb_fp_batch_obj: NULL argument");
+    REQUIRE(!eta || ((x && xk) || h->nvar == 0), FPSB_EINVAL, "fpsb_fp_batch_obj: eta needs x and xk");
+    FPB_RUN(fpb_obj(h, ninst, fx, rho, eta, c, ys, x, xk, phi))
+}
+int fpsb_fp_batch_grad(fpsb_handle hh, int64_t ninst, const double *sigma, const double *rho, const double *eta,
+                       const double *gs, const double *Hsv, const double *v, const double *Sstw, const double *Jtc,
+                       const double *x, const double *xk, double *g) {
+    FPB_BEGIN("fpsb_fp_batch_grad")
+    REQUIRE(sigma && gs && Hsv && v && Sstw && g, FPSB_EINVAL, "fpsb_fp_batch_grad: NULL argument");
+    REQUIRE(!rho || Jtc, FPSB_EINVAL, "fpsb_fp_batch_grad: rho needs J'c");
+    REQUIRE(!eta || (x && xk), FPSB_EINVAL, "fpsb_fp_batch_grad: eta needs x and xk");
+    FPB_RUN(fpb_grad(h, ninst, sigma, rho, eta, gs, Hsv, v, Sstw, Jtc, x, xk, g))
+}
+int fpsb_fp_batch_ptv(fpsb_handle hh, int64_t ninst, const double *v, const double *p1, double *Ptv) {
+    FPB_BEGIN("fpsb_fp_batch_ptv")
+    REQUIRE(v && p1 && Ptv, FPSB_EINVAL, "fpsb_fp_batch_ptv: NULL argument");
+    FPB_RUN(fpb_ptv(h, ninst, v, p1, Ptv))
+}
+int fpsb_fp_batch_hprod2(fpsb_handle hh, int64_t ninst, const double *sigma, const double *rho, const double *eta,
+                         const double *obj_weight, const double *p2, const double *HsPtv, const double *Ptv, const double *Hcv,
+                         const double *JtJv, const double *v, double *Hv) {
+    FPB_BEGIN("fpsb_fp_batch_hprod2")
+    REQUIRE(sigma && p2 && HsPtv && Ptv && v && Hv, FPSB_EINVAL, "fpsb_fp_batch_hprod2: NULL argument");
+    REQUIRE(!rho || (Hcv && JtJv), FPSB_EINVAL, "fpsb_fp_batch_hprod2: rho needs Hcv and J'Jv");
+    FPB_RUN(fpb_hprod2(h, ninst, sigma, rho, eta, obj_weight, p2, HsPtv, Ptv, Hcv, JtJv, v, Hv))
+}
+int fpsb_fp_batch_hprod1(fpsb_handle hh, int64_t ninst, const double *sigma, const double *rho, const double *eta,
+                         const double *obj_weight, const double *p2, const double *HsPtv, const double *Ptv,
+                         const double *JtinvJtJSsv, const double *SsinvJtJJv, const double *Hcv, const double *JtJv,
+                         const double *v, double *Hv) {
+    FPB_BEGIN("fpsb_fp_batch_hprod1")
+    REQUIRE(sigma && p2 && HsPtv && Ptv && JtinvJtJSsv && SsinvJtJJv && v && Hv, FPSB_EINVAL,
+            "fpsb_fp_batch_hprod1: NULL argument");
+    REQUIRE(!rho || (Hcv && JtJv), FPSB_EINVAL, "fpsb_fp_batch_hprod1: rho needs Hcv and J'Jv");
+    FPB_RUN(fpb_hprod1(h, ninst, sigma, rho, eta, obj_weight, p2, HsPtv, Ptv, JtinvJtJSsv, SsinvJtJJv, Hcv, JtJv, v, Hv))
+}
+int fpsb_batch_jprod(fpsb_handle hh, int64_t ninst, const double *jvals, int64_t jstride, const double *v, double *out) {
+    FPB_BEGIN("fpsb_batch_jprod")
+    REQUIRE(jstride == 0 || jstride == h->nnzj, FPSB_EINVAL, "fpsb_batch_jprod: jstride must be 0 or nnzj");
+    REQUIRE((jvals || h->nnzj == 0) && (v || h->nvar == 0) && (out || h->ncon == 0), FPSB_EINVAL,
+            "fpsb_batch_jprod: NULL argument");
+    FPB_RUN(fpb_spmv(h, false, ninst, jvals, jstride, v, out))
+}
+int fpsb_batch_jtprod(fpsb_handle hh, int64_t ninst, const double *jvals, int64_t jstride, const double *u, double *out) {
+    FPB_BEGIN("fpsb_batch_jtprod")
+    REQUIRE(jstride == 0 || jstride == h->nnzj, FPSB_EINVAL, "fpsb_batch_jtprod: jstride must be 0 or nnzj");
+    REQUIRE((jvals || h->nnzj == 0) && (u || h->ncon == 0) && (out || h->nvar == 0), FPSB_EINVAL,
+            "fpsb_batch_jtprod: NULL argument");
+    FPB_RUN(fpb_spmv(h, true, ninst, jvals, jstride, u, out))
+}
+int fpsb_trcg_batch_init(fpsb_handle hh, int64_t ninst, const double *g, const double *free_mask, const double *tol,
+                         double *s, double *r, double *d, double *st, int32_t *nprod, int32_t *nactive) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQUIRE(h && nactive, FPSB_EINVAL, "fpsb_trcg_batch_init: NULL argument");
+    REQUIRE(ninst >= 0, FPSB_EINVAL, "fpsb_trcg_batch_init: negative ninst");
+    *nactive = 0;
+    if (ninst == 0) return FPSB_OK;
+    REQUIRE(tol && st && nprod && ((g && s && r && d) || h->nvar == 0), FPSB_EINVAL, "fpsb_trcg_batch_init: NULL argument");
+    FPSB_TRY
+    FPSB_CUDA(cudaSetDevice(h->device));
+    caller_order_in(h);
+    *nactive = trcg_batch_init(h, ninst, g, free_mask, tol, s, r, d, st, nprod);
+    return FPSB_OK;
+    FPSB_CATCH
+}
+int fpsb_trcg_batch_step(fpsb_handle hh, int64_t ninst, const double *Hd, const double *free_mask, const double *radius,
+                         const double *tol, double *s, double *r, double *d, double *st, int32_t *nprod, int32_t *nactive) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQUIRE(h && nactive, FPSB_EINVAL, "fpsb_trcg_batch_step: NULL argument");
+    REQUIRE(ninst >= 0, FPSB_EINVAL, "fpsb_trcg_batch_step: negative ninst");
+    *nactive = 0;
+    if (ninst == 0) return FPSB_OK;
+    REQUIRE(radius && tol && st && nprod && ((Hd && s && r && d) || h->nvar == 0), FPSB_EINVAL,
+            "fpsb_trcg_batch_step: NULL argument");
+    FPSB_TRY
+    FPSB_CUDA(cudaSetDevice(h->device));
+    caller_order_in(h);
+    *nactive = trcg_batch_step(h, ninst, Hd, free_mask, radius, tol, s, r, d, st, nprod);
+    return FPSB_OK;
+    FPSB_CATCH
+}
+
 }  // extern "C"

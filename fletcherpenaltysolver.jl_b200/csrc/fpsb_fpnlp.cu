@@ -9,6 +9,8 @@
 //   grad!             gs - Hsv + sigma v + Sstw (+ rho J'c) (+ eta (x - xk))    :382-398
 //   hprod! (Val 2)    Ptv = v - p1 ; Hv = p2 - HsPtv + 2 sigma Ptv (+ Hcv + rho J'Jv) (+ eta v), times obj_weight   :543-568
 // All pointers are DEVICE pointers; scalar results come back through a pinned host slot.
+// The batched forms (many instances of one model, fpsb_fp_batch_*, fpsb_batch_j*prod, fpsb_trcg_batch_*) are in
+// fpsb_fpnlp_batch.inl, included at the end.
 #include "fpsb_internal.h"
 #include "fpsb_device.cuh"
 
@@ -220,7 +222,8 @@ struct FpWs {
     DevBuf<double> partials, out, trcg;
     DevBuf<unsigned> counter;
     DevBuf<unsigned long long> key;
-    double *h_out = nullptr;               // pinned: 3 doubles + 1 u64
+    DevBuf<unsigned> bcount;               // batched CG: instances still going
+    double *h_out = nullptr;               // pinned: 3 doubles + 1 u64 + 1 u32 (batched CG count, at double 6)
 };
 
 static FpWs *fp_ws(Handle *h) {
@@ -233,6 +236,7 @@ static FpWs *fp_ws(Handle *h) {
         W->counter.alloc(4);
         W->key.alloc(2);
         W->counter.zero(h->stream);
+        W->bcount.alloc(1);
         FPSB_CUDA(cudaMallocHost((void **)&W->h_out, 8 * sizeof(double)));
         h->fp = W;
     }
@@ -330,5 +334,7 @@ uint64_t fp_hash(Handle *h, int64_t n, const double *x) {
     FPSB_CUDA(cudaStreamSynchronize(h->stream));
     return (uint64_t)*hk;
 }
+
+#include "fpsb_fpnlp_batch.inl"
 
 }  // namespace fpsb

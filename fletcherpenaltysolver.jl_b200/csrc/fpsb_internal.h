@@ -167,6 +167,9 @@ void iter_solve_two_extras(Handle *h, double delta, const double *rhs1, const do
 void extras_batch(Handle *h, int64_t ninst, const double *jvals, const double *delta, const double *rhs1,
                   const double *rhs2, double *u1, double *u2, fpsb_krylov_stats *stats, const fpsb_extras_opts *opts);
 void extras_free(Handle *h);
+// the plain CSR patterns of A and A' with the COO index of every slot, built at the first call (device, int):
+// rpA [m+1] | ciA [nnz] | pmA [nnz] | rpT [n+1] | ciT [nnz] | pmT [nnz]; used by extras_batch and fpb_spmv
+const int *jac_csr(Handle *h);
 
 // fpsb_dist.inl (row-partitioned Krylov over NCCL)
 void dist_unique_id(void *out128);
@@ -208,6 +211,27 @@ void trcg_init(Handle *h, int64_t n, const double *g, const double *fr, double *
 void trcg_step(Handle *h, int64_t n, const double *Hd, const double *fr, double *s, double *r, double *d, double radius, double tol,
                double *out5);
 uint64_t fp_hash(Handle *h, int64_t n, const double *x);
+// fpsb_fpnlp_batch.inl: the same for `ninst` instances ([ninst][n] / [ninst][m] vectors, [ninst] scalar arrays)
+void fpb_ys_gs(Handle *h, int64_t ninst, const double *sigma, const double *p1, const double *q1, const double *p2,
+               const double *q2, double *gs, double *ys, double *v, double *w);
+void fpb_hash(Handle *h, int64_t ninst, const double *x, uint64_t *keys);
+void fpb_obj(Handle *h, int64_t ninst, const double *fx, const double *rho, const double *eta, const double *c,
+             const double *ys, const double *x, const double *xk, double *phi);
+void fpb_grad(Handle *h, int64_t ninst, const double *sigma, const double *rho, const double *eta, const double *gs,
+              const double *Hsv, const double *v, const double *Sstw, const double *Jtc, const double *x, const double *xk,
+              double *g);
+void fpb_ptv(Handle *h, int64_t ninst, const double *v, const double *p1, double *Ptv);
+void fpb_hprod2(Handle *h, int64_t ninst, const double *sigma, const double *rho, const double *eta, const double *obj_weight,
+                const double *p2, const double *HsPtv, const double *Ptv, const double *Hcv, const double *JtJv,
+                const double *v, double *Hv);
+void fpb_hprod1(Handle *h, int64_t ninst, const double *sigma, const double *rho, const double *eta, const double *obj_weight,
+                const double *p2, const double *HsPtv, const double *Ptv, const double *JtinvJtJSsv,
+                const double *SsinvJtJJv, const double *Hcv, const double *JtJv, const double *v, double *Hv);
+void fpb_spmv(Handle *h, bool transpose, int64_t ninst, const double *jvals, int64_t jstride, const double *x, double *out);
+int32_t trcg_batch_init(Handle *h, int64_t ninst, const double *g, const double *fr, const double *tol, double *s, double *r,
+                        double *d, double *st, int *nprod);
+int32_t trcg_batch_step(Handle *h, int64_t ninst, const double *Hd, const double *fr, const double *radius, const double *tol,
+                        double *s, double *r, double *d, double *st, int *nprod);
 
 // symbolic.cpp / ldlt.cu
 void ldlt_analyze(Handle *h, const int64_t *P, const fpsb_ldlt_opts *opts);

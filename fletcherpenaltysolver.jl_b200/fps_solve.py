@@ -438,6 +438,49 @@ def _steihaug_device(handle, hv, g, radius, tol, itmax, free=None):
     return s, -out[1], nprod
 
 
+def _steihaug_batch(handle, hv, G, radius, tol, itmax, free=None):
+    """`_steihaug_device` for K subproblems in lock-step: instance i is  min G[i]'s + s'H_i s/2, ‖s‖ ≤ radius[i], and
+    `hv(D)` returns the K products H_i D[i] as one (K, n) tensor (one batched `hprod`).  radius and tol are scalars or
+    (K,); free is None or (K, n).  Each instance runs inside one CTA of fpsb_trcg_batch_step; an instance that has left
+    (boundary, negative curvature, converged) is frozen while the others keep going, and its rows of the later products
+    are computed with the batch and discarded, so `hv` always sees the full batch.  The host reads one 4-byte count of
+    active instances per iteration.  Returns S (K, n), pred (K,) (the model decrease −q), nprod (K,) int32 and the exit
+    flags (K,): 0 itmax reached, 1 left through the boundary or met non-positive curvature, 2 converged (also for a
+    gradient with ‖g‖ ≤ tol, with no product)."""
+    import ctypes as C
+    import torch
+    from . import _lib
+    L = _lib.lib()
+    if G.ndim != 2 or G.shape[1] != handle.nvar:
+        raise ValueError(f"_steihaug_batch: G must be (K, {handle.nvar})")
+    K = int(G.shape[0])
+    G = G.to(torch.float64).contiguous()
+    f64 = dict(dtype=torch.float64, device=G.device)
+    per = lambda a: torch.as_tensor(a, **f64).expand(K).contiguous()
+    rad, tl = per(radius), per(tol)
+    fr = None if free is None else free.to(torch.float64).contiguous()
+    if fr is not None and tuple(fr.shape) != tuple(G.shape):
+        raise ValueError("_steihaug_batch: free must have the shape of G")
+    S, R, D = torch.empty_like(G), torch.empty_like(G), torch.empty_like(G)
+    st = torch.zeros((K, 5), **f64)
+    nprod = torch.zeros(K, dtype=torch.int32, device=G.device)
+    if K == 0:
+        return S, st[:, 1], nprod, st[:, 4]
+    handle._follow_torch_stream(G)
+    p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+    nact = C.c_int32()
+    _lib.check(L.fpsb_trcg_batch_init(handle.h, C.c_int64(K), p(G), p(fr), p(tl), p(S), p(R), p(D), p(st), p(nprod),
+                                      C.byref(nact)), "fpsb_trcg_batch_init")
+    it = 0
+    while nact.value > 0 and it < itmax:
+        Hd = hv(D).to(torch.float64).contiguous()
+        it += 1
+        handle._follow_torch_stream(Hd)
+        _lib.check(L.fpsb_trcg_batch_step(handle.h, C.c_int64(K), p(Hd), p(fr), p(rad), p(tl), p(S), p(R), p(D), p(st),
+                                          p(nprod), C.byref(nact)), "fpsb_trcg_batch_step")
+    return S, -st[:, 1], nprod, st[:, 4].clone()
+
+
 def _cg_solver_for(model, g):
     """The device-resident CG when the iterate lives on the GPU and the model owns a libfpsb200 handle, else the host loop."""
     h = getattr(model, "handle", None)

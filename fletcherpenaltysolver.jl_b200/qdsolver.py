@@ -138,6 +138,38 @@ class B200Handle:
     def jtprod(self, u):
         return self._spmv(_lib.lib().fpsb_jtprod, u, self.nvar)
 
+    def _batch_spmv(self, fn, name, jvals, X, nin, nout):
+        import torch
+        if not (hasattr(X, "is_cuda") and X.is_cuda):
+            raise TypeError(f"{name}: expects CUDA tensors")
+        X = X.to(torch.float64).contiguous()
+        jvals = torch.as_tensor(jvals, dtype=torch.float64, device=X.device).contiguous()
+        if X.ndim != 2 or X.shape[1] != nin:
+            raise ValueError(f"{name}: the vectors must be (ninst, {nin})")
+        ninst = int(X.shape[0])
+        if tuple(jvals.shape) == (self.nnzj,):
+            stride = 0
+        elif tuple(jvals.shape) == (ninst, self.nnzj):
+            stride = self.nnzj
+        else:
+            raise ValueError(f"{name}: jvals must be ({self.nnzj},) or (ninst, {self.nnzj})")
+        out = torch.empty((ninst, nout), dtype=torch.float64, device=X.device)
+        if ninst == 0:
+            return out
+        self._follow_torch_stream(X)
+        check(fn(self.h, C.c_int64(ninst), C.c_void_p(jvals.data_ptr()), C.c_int64(stride), C.c_void_p(X.data_ptr()),
+                 C.c_void_p(out.data_ptr())), name)
+        return out
+
+    def batch_jprod(self, jvals, V):
+        """A_i v_i for every row of V (ninst, nvar) -> (ninst, ncon), A_i with the values jvals[i] (COO order of this
+        handle's pattern); jvals (nnzj,) is one set of values for every instance (fpsb_batch_jprod).  CUDA tensors."""
+        return self._batch_spmv(_lib.lib().fpsb_batch_jprod, "fpsb_batch_jprod", jvals, V, self.nvar, self.ncon)
+
+    def batch_jtprod(self, jvals, U):
+        """A_i' u_i for every row of U (ninst, ncon) -> (ninst, nvar) (fpsb_batch_jtprod); jvals as in batch_jprod."""
+        return self._batch_spmv(_lib.lib().fpsb_batch_jtprod, "fpsb_batch_jtprod", jvals, U, self.ncon, self.nvar)
+
     def jprod2(self, v):
         return self._spmv(_lib.lib().fpsb_jprod2, v, self.ncon, 2)
 

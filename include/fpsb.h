@@ -384,6 +384,61 @@ int fpsb_fp_hprod1(fpsb_handle h, double sigma, double rho, double eta, double o
                    const double *HsPtv, const double *Ptv, const double *JtinvJtJSsv, const double *SsinvJtJJv,
                    const double *Hcv, const double *JtJv, const double *v, double *Hv);
 
+/* ---------------------------------------------------------------------------------------------
+ * Batched FletcherPenaltyNLP glue: the entries above for `ninst` instances of ONE model (one handle), each at its own
+ * point with its own sigma, rho, eta, xk and Jacobian values.  ALL arguments are DEVICE pointers; vectors are
+ * instance-major, [ninst][nvar] or [ninst][ncon]; per-instance scalars are arrays [ninst].  rho, eta and obj_weight may
+ * be NULL, which reads as 0 (obj_weight: 1) for every instance; a non-NULL rho needs its J'c / Hcv and J'Jv arguments
+ * and a non-NULL eta needs x and xk, else FPSB_EINVAL (the checks of the single entries, made on the host without
+ * reading the arrays).  The element-wise entries evaluate the single kernel's expression in its operation order, so
+ * every entry is bitwise what the single entry gives on the same inputs; per-instance sums run inside one CTA, so
+ * results do not depend on ninst or on an instance's position in the batch.  ninst == 0 is a no-op, a negative ninst
+ * FPSB_EINVAL.  Asynchronous and ordered against the caller's stream (fpsb_set_caller_stream), except the CG entries,
+ * which return after one 4-byte read-back.  None of them touches the handle's single-instance Jacobian values, Krylov
+ * workspaces or the factors of fpsb_ldlt_batch_solve_two_mixed (Val(1): mixed -> least squares -> extras -> products).
+ *   fpsb_fp_batch_ys_gs   fpsb_fp_ys_gs per instance                                  src/model-Fletcherpenaltynlp.jl:244-248
+ *   fpsb_fp_batch_hash    keys [ninst] (device): key i is bit for bit fpsb_fp_hash of row i                     :235
+ *   fpsb_fp_batch_obj     phi [ninst] (device) = fx - c'ys + rho/2 |c|^2 (+ eta/2 |x - xk|^2), fx [ninst]  :364-367
+ *   fpsb_fp_batch_grad    fpsb_fp_grad per instance                                                     :382-398
+ *   fpsb_fp_batch_ptv     fpsb_fp_ptv per instance                                                          :544
+ *   fpsb_fp_batch_hprod2  fpsb_fp_hprod2 per instance, obj_weight [ninst]                               :546-568
+ *   fpsb_fp_batch_hprod1  fpsb_fp_hprod1 per instance, obj_weight [ninst]                               :572-634
+ *   fpsb_batch_jprod      out_i = A_i v_i  [ninst][ncon]  (jprod! of the rho-terms, :560-566; cons of linear models)
+ *   fpsb_batch_jtprod     out_i = A_i' u_i [ninst][nvar]  (jtprod! of J'c :390, J'Jv :566, Val(1) :612)
+ *                         jvals + i * jstride holds instance i's values in the COO order given to fpsb_create;
+ *                         jstride is nnzj, or 0 when every instance shares one set of values.  One thread per output
+ *                         row sums in plain CSR order, so results differ from fpsb_jprod / fpsb_jtprod (tiled SELL-32)
+ *                         in the last bits. */
+int fpsb_fp_batch_ys_gs(fpsb_handle h, int64_t ninst, const double *sigma, const double *p1, const double *q1,
+                        const double *p2, const double *q2, double *gs, double *ys, double *v, double *w);
+int fpsb_fp_batch_hash(fpsb_handle h, int64_t ninst, const double *x, uint64_t *keys);
+int fpsb_fp_batch_obj(fpsb_handle h, int64_t ninst, const double *fx, const double *rho, const double *eta, const double *c,
+                      const double *ys, const double *x, const double *xk, double *phi);
+int fpsb_fp_batch_grad(fpsb_handle h, int64_t ninst, const double *sigma, const double *rho, const double *eta,
+                       const double *gs, const double *Hsv, const double *v, const double *Sstw, const double *Jtc,
+                       const double *x, const double *xk, double *g);
+int fpsb_fp_batch_ptv(fpsb_handle h, int64_t ninst, const double *v, const double *p1, double *Ptv);
+int fpsb_fp_batch_hprod2(fpsb_handle h, int64_t ninst, const double *sigma, const double *rho, const double *eta,
+                         const double *obj_weight, const double *p2, const double *HsPtv, const double *Ptv, const double *Hcv,
+                         const double *JtJv, const double *v, double *Hv);
+int fpsb_fp_batch_hprod1(fpsb_handle h, int64_t ninst, const double *sigma, const double *rho, const double *eta,
+                         const double *obj_weight, const double *p2, const double *HsPtv, const double *Ptv,
+                         const double *JtinvJtJSsv, const double *SsinvJtJJv, const double *Hcv, const double *JtJv,
+                         const double *v, double *Hv);
+int fpsb_batch_jprod(fpsb_handle h, int64_t ninst, const double *jvals, int64_t jstride, const double *v, double *out);
+int fpsb_batch_jtprod(fpsb_handle h, int64_t ninst, const double *jvals, int64_t jstride, const double *u, double *out);
+/* Batched Steihaug-Toint CG (fpsb_trcg_init / fpsb_trcg_step per instance, one CTA per instance, one kernel per
+ * iteration).  g, free_mask (nullable), s, r, d, Hd [ninst][nvar]; radius, tol [ninst]; st [ninst][5] = {rr, q, tau,
+ * beta, flag} as `out` of the single entry, except that init already sets flag 2 when sqrt(rr) <= tol (zero step, no
+ * product); nprod [ninst] (int32) counts the products each instance consumed.  An instance whose flag is non-zero is
+ * frozen: its s, r, d, st and nprod are not touched again, so the caller keeps computing Hd for the whole batch and
+ * ignores the frozen rows.  *nactive (host) receives the number of instances still going: the one host
+ * synchronisation per iteration of the whole batch. */
+int fpsb_trcg_batch_init(fpsb_handle h, int64_t ninst, const double *g, const double *free_mask, const double *tol,
+                         double *s, double *r, double *d, double *st, int32_t *nprod, int32_t *nactive);
+int fpsb_trcg_batch_step(fpsb_handle h, int64_t ninst, const double *Hd, const double *free_mask, const double *radius,
+                         const double *tol, double *s, double *r, double *d, double *st, int32_t *nprod, int32_t *nactive);
+
 #ifdef __cplusplus
 }
 #endif

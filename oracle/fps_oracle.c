@@ -920,6 +920,17 @@ void fo_lsqr_csr(i64 m, i64 n, const i64 *rp, const i64 *ci, const double *vx,
     fo_op op = { &M, kind, NULL };
     fo_lsqr(&op, b, lambda, atol, rtol, SQRT_EPS, SQRT_EPS, SQRT_EPS, 1.0 / SQRT_EPS, itmax, x, st);
 }
+/* LSQR with every threshold settable (fo_lsqr_csr fixes axtol = btol = etol = sqrt(eps) and conlim = 1/sqrt(eps),
+   as the reference's call site does); tests scale them to show that a stopping decision is not a near tie */
+void fo_lsqr_full_csr(i64 m, i64 n, const i64 *rp, const i64 *ci, const double *vx,
+                      const i64 *trp, const i64 *tci, const double *tvx, int kind,
+                      const double *b, double lambda, double atol, double rtol, double axtol, double btol,
+                      double etol, double conlim, i64 itmax, double *x, fo_stats *st)
+{
+    fo_mat M; mk_mat(&M, m, n, rp, ci, vx, trp, tci, tvx);
+    fo_op op = { &M, kind, NULL };
+    fo_lsqr(&op, b, lambda, atol, rtol, axtol, btol, etol, conlim, itmax, x, st);
+}
 void fo_craig_csr(i64 m, i64 n, const i64 *rp, const i64 *ci, const double *vx,
                   const i64 *trp, const i64 *tci, const double *tvx, int kind,
                   const double *b, int sqd, double mscale, double atol, double rtol, double btol,

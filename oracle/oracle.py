@@ -186,12 +186,15 @@ class _Mat:
                 _p(self.trp), _p(self.tci), _p(self.tvx))
 
 
-def lsqr(A, b, lam=0.0, atol=SQRT_EPS, rtol=SQRT_EPS, itmax=0, transpose=False):
-    """Krylov.lsqr on A (transpose=False) or A' (True) with the reference's call-site kwargs."""
+def lsqr(A, b, lam=0.0, atol=SQRT_EPS, rtol=SQRT_EPS, itmax=0, transpose=False, axtol=SQRT_EPS,
+         btol=SQRT_EPS, etol=SQRT_EPS, conlim=1 / SQRT_EPS):
+    """Krylov.lsqr on A (transpose=False) or A' (True); the defaults are the reference's call-site kwargs
+    (axtol, btol, etol and conlim are Krylov.jl's defaults, which that call site does not override)."""
     M = _Mat(A); b = _f64(b)
     x = np.zeros(M.m if transpose else M.n); st = Stats()
-    lib().fo_lsqr_csr(*M.args(), C.c_int(1 if transpose else 0), _p(b), C.c_double(lam),
-                      C.c_double(atol), C.c_double(rtol), C.c_int64(itmax), _p(x), C.byref(st))
+    lib().fo_lsqr_full_csr(*M.args(), C.c_int(1 if transpose else 0), _p(b), C.c_double(lam),
+                           C.c_double(atol), C.c_double(rtol), C.c_double(axtol), C.c_double(btol),
+                           C.c_double(etol), C.c_double(conlim), C.c_int64(itmax), _p(x), C.byref(st))
     return x, st.as_dict()
 
 

@@ -53,7 +53,7 @@ class ExtrasOpts(C.Structure):
 EXPORTS = [
     "fpsb_version", "fpsb_last_error", "fpsb_device_count", "fpsb_create", "fpsb_destroy",
     "fpsb_dims", "fpsb_pin_host", "fpsb_unpin_host", "fpsb_stream", "fpsb_set_caller_stream", "fpsb_synchronize", "fpsb_timer_start", "fpsb_timer_stop",
-    "fpsb_launch_count", "fpsb_pipeline_gate", "fpsb_tile_stats", "fpsb_set_jac_values", "fpsb_jprod", "fpsb_jtprod", "fpsb_jprod2",
+    "fpsb_launch_count", "fpsb_pipeline_gate", "fpsb_tile_stats", "fpsb_tile_layout", "fpsb_tile_segments", "fpsb_set_jac_values", "fpsb_jprod", "fpsb_jtprod", "fpsb_jprod2",
     "fpsb_jtprod2", "fpsb_iter_default_opts", "fpsb_iter_setup", "fpsb_iter_solve_two_mixed",
     "fpsb_iter_solve_two_least_squares", "fpsb_iter_solve_two_extras", "fpsb_iter_last_profile", "fpsb_iter_loop_info", "fpsb_ldlt_default_opts",
     "fpsb_ldlt_analyze", "fpsb_ldlt_symbolic_sizes", "fpsb_ldlt_get_symbolic",

@@ -255,6 +255,30 @@ int fpsb_tile_stats(fpsb_handle hh, int64_t out[6]) {
     out[3] = h->At.ntiles; out[4] = h->At.nwin_tiles; out[5] = h->At.nseg_tiles;
     return FPSB_OK;
 }
+int fpsb_tile_layout(fpsb_handle hh, int64_t out[16]) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQUIRE(h && out, FPSB_EINVAL, "fpsb_tile_layout: NULL argument");
+    const CsrDev *ops[2] = {&h->A, &h->At};
+    for (int i = 0; i < 2; ++i) {
+        const CsrDev &M = *ops[i];
+        int64_t *o = out + 8 * i;
+        o[0] = M.ntiles; o[1] = M.nwin_tiles; o[2] = M.nseg_tiles; o[3] = M.nglob_tiles;
+        o[4] = M.nodd_tiles; o[5] = M.nlong; o[6] = M.nns0_tiles; o[7] = M.nmixed_tiles;
+    }
+    return FPSB_OK;
+}
+int fpsb_tile_segments(fpsb_handle hh, int transpose, int64_t tile, int64_t out[8]) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQUIRE(h && out, FPSB_EINVAL, "fpsb_tile_segments: NULL argument");
+    const CsrDev &M = transpose ? h->At : h->A;
+    REQUIRE(tile >= 0 && tile < M.ntiles, FPSB_EINVAL, "fpsb_tile_segments: tile out of range");
+    for (int g = 0; g < 4; ++g) {
+        const bool have = !M.wsegs_host.empty();
+        out[2 * g] = have ? M.wsegs_host[(size_t)(tile * 4 + g) * 2] : 0;
+        out[2 * g + 1] = have ? (M.wsegs_host[(size_t)(tile * 4 + g) * 2 + 1] >> 16) : 0;
+    }
+    return FPSB_OK;
+}
 
 int fpsb_set_jac_values(fpsb_handle hh, const double *vals, int loc) {
     Handle *h = reinterpret_cast<Handle *>(hh);

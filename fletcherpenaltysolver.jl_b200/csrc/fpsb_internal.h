@@ -70,6 +70,10 @@ struct CsrDev {
     bool has_raw_rows = false;
     DevBuf<int> wsegs;                         // multi-segment gather windows: 4 x {start, offset | length << 16} per tile
     int nseg_tiles = 0, nwin_tiles = 0;        // tiles whose window has more than one segment / tiles with a window at all
+    // layout counters (fpsb_tile_layout): tiles without a window (global int32 indices), with an odd window length,
+    // without any slice (every row long), holding long rows next to their slices (nsell < nrows)
+    int nglob_tiles = 0, nodd_tiles = 0, nns0_tiles = 0, nmixed_tiles = 0;
+    std::vector<int> wsegs_host;               // host copy of wsegs (fpsb_tile_segments); empty without multi-segment tiles
     int ntiles = 0, win_cap = 0, blk_cap = 0, stage_bytes = 0, nstage = 0;
     DevBuf<int> long_row, long_rp, long_col, long_perm;
     DevBuf<double> long_val;

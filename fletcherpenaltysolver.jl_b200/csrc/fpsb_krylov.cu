@@ -1679,6 +1679,8 @@ static void upload_sell(Handle *h, CsrDev &M, int nrows, int ncols, const std::v
                         const std::vector<int> &ci, const std::vector<int> &perm) {
     M.nrows = nrows; M.ncols = ncols; M.nnz = (int64_t)ci.size();
     M.nseg_tiles = M.nwin_tiles = 0;
+    M.nglob_tiles = M.nodd_tiles = M.nns0_tiles = M.nmixed_tiles = 0;
+    M.wsegs_host.clear();
     std::vector<int> long_row, long_rp(1, 0), long_col, long_perm;
     std::vector<unsigned char> rowflag((size_t)nrows + 8, 0);
     std::vector<TileMeta> tiles;
@@ -1821,7 +1823,10 @@ static void upload_sell(Handle *h, CsrDev &M, int nrows, int ncols, const std::v
             std::array<Seg, kMaxSeg> sg{};
             if (!segs.empty()) { for (size_t g = 0; g < segs.size(); ++g) sg[g] = segs[g]; ++M.nseg_tiles; }
             else if (cnt > 0) sg[0] = Seg{c0, cnt};
-            if (cnt > 0) ++M.nwin_tiles;
+            if (cnt > 0) ++M.nwin_tiles; else ++M.nglob_tiles;
+            if (cnt & 1) ++M.nodd_tiles;
+            if (T.ns == 0) ++M.nns0_tiles;
+            if (T.nsell < T.nrows) ++M.nmixed_tiles;
             tile_segs.push_back(sg);
         }
         tperm0.push_back((int)total_elems);
@@ -1928,6 +1933,7 @@ static void upload_sell(Handle *h, CsrDev &M, int nrows, int ncols, const std::v
             }
         }
         M.wsegs.from(ws, h->stream);
+        M.wsegs_host.swap(ws);
     }
     M.long_row.from(long_row, h->stream);
     M.long_rp.from(long_rp, h->stream);

@@ -112,6 +112,23 @@ class B200Handle:
         return {"A": dict(tiles=v[0], windowed=v[1], multi_segment=v[2]),
                 "At": dict(tiles=v[3], windowed=v[4], multi_segment=v[5])}
 
+    LAYOUT_KEYS = ("tiles", "windowed", "multi_segment", "global", "odd_window", "long_rows", "no_slices", "mixed")
+
+    def tile_layout(self):
+        """Per operator (A, A'): tiles, windowed / multi-segment / global-index tiles, odd-window tiles, long rows,
+        tiles without slices and tiles mixing long rows with slices (fpsb_tile_layout)."""
+        out = (C.c_int64 * 16)()
+        check(_lib.lib().fpsb_tile_layout(self.h, out), "fpsb_tile_layout")
+        v = [int(x) for x in out]
+        return {"A": dict(zip(self.LAYOUT_KEYS, v[:8])), "At": dict(zip(self.LAYOUT_KEYS, v[8:]))}
+
+    def tile_segments(self, tile, transpose=False):
+        """[(start column, length), ...] of the gather-window segments of one tile (fpsb_tile_segments); empty when
+        the operator has no multi-segment tile."""
+        out = (C.c_int64 * 8)()
+        check(_lib.lib().fpsb_tile_segments(self.h, C.c_int(int(transpose)), C.c_int64(tile), out), "fpsb_tile_segments")
+        return [(int(out[2 * g]), int(out[2 * g + 1])) for g in range(4) if out[2 * g + 1] > 0]
+
     # -- Jacobian ------------------------------------------------------------------------------
     def set_jac_values(self, vals):
         if isinstance(vals, np.ndarray):

@@ -120,6 +120,16 @@ int64_t fpsb_launch_count(fpsb_handle h);
  * LinearOperator `jac_op!`, src/solve_linear_system.jl:119-121): out = {tiles of A, of those with a shared-memory gather
  * window, of those with a multi-segment window (stencil operators), the same three for A'}. */
 int fpsb_tile_stats(fpsb_handle h, int64_t out[6]);
+/* Finer layout of the same operators, out[0..7] for A and out[8..15] for A': {tiles, tiles with a window, tiles with a
+ * multi-segment window, tiles without a window (global int32 column indices), tiles with an odd window length, rows
+ * longer than the SELL limit (long-row kernel), tiles without any slice (every row long), tiles holding long rows
+ * next to their slices}.  Host only: touches nothing on the device. */
+int fpsb_tile_layout(fpsb_handle h, int64_t out[16]);
+/* The gather-window segments of one tile of A (transpose = 0) or A' (transpose = 1) on an operator that has
+ * multi-segment tiles: out = {start column, length} of up to four column runs copied back to back, unused ones zero.
+ * A single-window tile reports its one run, a tile without a window zeros; all zero when the operator has no
+ * multi-segment tile.  Host only. */
+int fpsb_tile_segments(fpsb_handle h, int transpose, int64_t tile, int64_t out[8]);
 
 /* Replaces jac_coord!(nlp, x, vals[nvar+1 : nvar+nnzj]) feeding both paths
  *   src/solve_linear_system.jl:224-228 (LDLt)  and  jac_op! at :119-121 (Iterative).

@@ -49,6 +49,29 @@ def test_argument_validation():
         SymbolicAnalysis(3, 2, [0, 1], [0, 2], P=[0, 0, 1, 2, 3])
 
 
+def test_tile_layout_and_create_validation():
+    """fpsb_tile_layout and fpsb_tile_segments reject a NULL handle and a NULL output; fpsb_create rejects an
+    out-of-range index before it looks for a device."""
+    L = _lib.lib()
+    out = (ctypes.c_int64 * 16)()
+    assert L.fpsb_tile_layout(None, out) == -1 and b"NULL" in L.fpsb_last_error()
+    fake = ctypes.create_string_buffer(64)
+    assert L.fpsb_tile_layout(ctypes.cast(fake, ctypes.c_void_p), None) == -1
+    seg = (ctypes.c_int64 * 8)()
+    assert L.fpsb_tile_segments(None, 0, ctypes.c_int64(0), seg) == -1
+    assert L.fpsb_tile_segments(ctypes.cast(fake, ctypes.c_void_p), 0, ctypes.c_int64(0), None) == -1
+    h = ctypes.c_void_p()
+    for r, c in (([2], [0]), ([0], [4]), ([-1], [0])):
+        jr, jc = np.array(r, dtype=np.int64), np.array(c, dtype=np.int64)
+        rc = L.fpsb_create(ctypes.c_int64(4), ctypes.c_int64(2), ctypes.c_int64(1), jr.ctypes.data_as(ctypes.c_void_p),
+                           jc.ctypes.data_as(ctypes.c_void_p), ctypes.c_int(0), ctypes.c_int(0), ctypes.byref(h))
+        assert rc == -1 and b"out of range" in L.fpsb_last_error() and not h.value
+    jr = np.array([0], dtype=np.int64)           # one-based: 0 is out of range
+    rc = L.fpsb_create(ctypes.c_int64(4), ctypes.c_int64(2), ctypes.c_int64(1), jr.ctypes.data_as(ctypes.c_void_p),
+                       jr.ctypes.data_as(ctypes.c_void_p), ctypes.c_int(1), ctypes.c_int(0), ctypes.byref(h))
+    assert rc == -1 and b"out of range" in L.fpsb_last_error()
+
+
 @pytest.mark.parametrize("m,n,k,w", [(1, 10, 9, 4), (30, 60, 5, 8), (500, 1000, 10, 32), (4000, 8000, 10, 64)])
 @pytest.mark.parametrize("pk", ["amd", "id", "rand"])
 def test_symbolic_bit_exact_vs_oracle(oracle, m, n, k, w, pk):

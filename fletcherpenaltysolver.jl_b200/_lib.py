@@ -42,6 +42,23 @@ class LdltOpts(C.Structure):
     _fields_ = [("ldlt_tol", C.c_double), ("ldlt_r1", C.c_double), ("ldlt_r2", C.c_double)]
 
 
+# fields of fpsb_symbolic_ldlt_routes / fpsb_ldlt_routes, in the order of include/fpsb.h
+LDLT_ROUTE_KEYS = (
+    "nsuper", "leaf1", "leaf_wide", "warp", "warp_nonleaf", "bundles", "full_bundles",
+    "cta", "cta_w64", "cta_w33_63", "max_nr", "trsm_multi", "solve_multi",
+    "upd_multi", "upd_nrow8", "upd_ncol8", "upd_wd4",
+    "leaf_contrib", "zero_slots", "multi_src", "levels",
+    "trsm_tail_m1", "trsm_tail_0", "trsm_tail_1", "solve_tail_m1", "solve_tail_0", "solve_tail_1",
+    "upd_tail_m1", "upd_tail_0", "upd_tail_1",
+)
+
+
+def ldlt_routes(fn, h, name):
+    out = (C.c_int64 * len(LDLT_ROUTE_KEYS))()
+    check(fn(h, out), name)
+    return dict(zip(LDLT_ROUTE_KEYS, (int(v) for v in out)))
+
+
 class ExtrasOpts(C.Structure):
     """fpsb_extras_opts — tolerances of the batched LDLt solve_two_extras (itmax 0 = Krylov.jl's default)."""
     _fields_ = [("cg_atol", C.c_double), ("cg_rtol", C.c_double), ("cg_itmax", C.c_int64),
@@ -61,7 +78,7 @@ EXPORTS = [
     "fpsb_ldlt_solve_two_mixed", "fpsb_ldlt_solve_two_least_squares", "fpsb_ldlt_solve_two_extras",
     "fpsb_ldlt_batch_solve_two_mixed", "fpsb_ldlt_batch_solve_two_least_squares", "fpsb_ldlt_batch_solve_two_extras",
     "fpsb_symbolic_create", "fpsb_symbolic_destroy", "fpsb_symbolic_sizes", "fpsb_symbolic_get",
-    "fpsb_symbolic_plan_info", "fpsb_order_dissection", "fpsb_batch_solve_two",
+    "fpsb_symbolic_plan_info", "fpsb_symbolic_ldlt_routes", "fpsb_ldlt_routes", "fpsb_order_dissection", "fpsb_batch_solve_two",
     "fpsb_dist_unique_id", "fpsb_dist_attach", "fpsb_dist_jprod", "fpsb_dist_jtprod",
     "fpsb_dist_solve_two_mixed", "fpsb_dist_solve_two_least_squares", "fpsb_dist_solve_two_extras", "fpsb_dist_profile", "fpsb_dist_last_profile",
     "fpsb_dist_peer_blob_bytes", "fpsb_dist_peer_export", "fpsb_dist_peer_attach", "fpsb_dist_peer_active",

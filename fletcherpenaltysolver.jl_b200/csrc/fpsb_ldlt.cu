@@ -1078,6 +1078,94 @@ __global__ void __launch_bounds__(kLdltBlock, 2) ldlt_batch_kernel(PlanDev P, Ba
 template <class T>
 static void up(DevBuf<T> &b, const std::vector<T> &v, cudaStream_t s) { b.from(v, s); }
 
+// the routine a supernode goes through: one warp (bundled with up to kWarpsPerBlock - 1 others) when it is this small,
+// a whole CTA otherwise; one-wide leaves go to leaf1_factor / leaf1_bwd whatever this says
+static bool warp_level(const Symbolic &S, int t) {
+    const int w = S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t];
+    const int nr = (int)(S.rptr[(size_t)t + 1] - S.rptr[(size_t)t]);
+    return w <= kSmallW && (int64_t)w * (w + nr) <= 512;
+}
+static bool leaf1(const Symbolic &S, int t) { return S.level[(size_t)t] == 0 && S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t] == 1; }
+
+// tasks of the single-instance launches: CTA-level supernodes alone (tcnt 0), warp-level ones bundled one per warp
+// (tcnt = bundle size), positions in S.order; tasks [0, ntasks_leaf) hold the leaves wider than one column
+static void build_tasks(const Symbolic &S, std::vector<int> &tstart, std::vector<int> &tcnt, int &ntasks_leaf) {
+    tstart.clear(); tcnt.clear();
+    // `order` is sorted by level: the first nleaf entries are the leaf supernodes; bundles never
+    // straddle the leaf / non-leaf boundary (they are processed by different launches)
+    for (int part = 0; part < 2; part++) {
+        int i = part == 0 ? 0 : S.nleaf;
+        const int end = part == 0 ? S.nleaf : S.nsuper;
+        while (i < end) {
+            if (leaf1(S, S.order[(size_t)i])) { i++; continue; }      // leaf1_*_kernel
+            if (warp_level(S, S.order[(size_t)i])) {
+                int j = i;
+                while (j < end && j - i < kWarpsPerBlock && warp_level(S, S.order[(size_t)j]) && !leaf1(S, S.order[(size_t)j])) j++;
+                tstart.push_back(i); tcnt.push_back(j - i);
+                i = j;
+            } else {
+                tstart.push_back(i); tcnt.push_back(0);
+                i++;
+            }
+        }
+        if (part == 0) ntasks_leaf = (int)tstart.size();
+    }
+}
+
+// fpsb_ldlt_routes / fpsb_symbolic_ldlt_routes: which routine and which staging passes each supernode and update pair
+// of the plan go through, from the predicates the launches use (field order: include/fpsb.h)
+static void ldlt_routes(const Symbolic &S, int64_t *out) {
+    for (int k = 0; k < FPSB_LDLT_ROUTES; ++k) out[k] = 0;
+    std::vector<int> tstart, tcnt;
+    int ntl = 0;
+    build_tasks(S, tstart, tcnt, ntl);
+    auto nr_of = [&](int t) { return (int)(S.rptr[(size_t)t + 1] - S.rptr[(size_t)t]); };
+    auto w_of = [&](int t) { return S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t]; };
+    auto tail = [](int64_t *o, int n, int pass) {            // the last pass one row short of full, full, one row
+        if (n <= 0) return;
+        const int r = n % pass;
+        if (r == pass - 1) o[0]++;
+        else if (r == 0) o[1]++;
+        else if (r == 1 && n > pass) o[2]++;
+    };
+    out[0] = S.nsuper;
+    int64_t lower = 0;
+    for (int t = 0; t < S.nsuper; ++t) {
+        const int w = w_of(t), nr = nr_of(t);
+        if (leaf1(S, t)) out[1]++;
+        else if (S.level[(size_t)t] == 0) out[2]++;
+        if (!leaf1(S, t) && warp_level(S, t)) { out[3]++; if (S.level[(size_t)t] > 0) out[4]++; }
+        out[10] = std::max<int64_t>(out[10], nr);
+        lower += (int64_t)w * (w + 1) / 2 + (int64_t)w * nr;
+    }
+    for (size_t k = 0; k < tstart.size(); ++k) {
+        if (tcnt[k] > 0) { out[5]++; if (tcnt[k] == kWarpsPerBlock) out[6]++; continue; }
+        if ((int)k < ntl) continue;                          // wider leaves: scalar CTA routines in every mode
+        const int t = S.order[(size_t)tstart[k]];
+        const int w = w_of(t), nr = nr_of(t);
+        out[7]++;
+        if (w == kMaxW) out[8]++;
+        else if (w > 32) out[9]++;
+        if (nr > kTrsmRows) out[11]++;
+        if (nr > kSolveRows) out[12]++;
+        tail(out + 21, nr, kTrsmRows);
+        tail(out + 24, nr, kSolveRows);
+        for (int64_t q = S.uptr[(size_t)t]; q < S.umid[(size_t)t]; ++q) {
+            const int d = S.usrc[(size_t)q];
+            const int nrow = nr_of(d) - S.ua[(size_t)q], ncol = S.ub[(size_t)q] - S.ua[(size_t)q];
+            if (nrow > kUpdRows) out[13]++;
+            if (nrow % 8) out[14]++;
+            if (ncol % 8) out[15]++;
+            if (w_of(d) % 4) out[16]++;
+            tail(out + 27, nrow, kUpdRows);
+        }
+    }
+    out[17] = S.lcptr.empty() ? 0 : S.lcptr[(size_t)S.N];
+    out[18] = lower - (S.N + (S.Lp.empty() ? 0 : S.Lp[(size_t)S.N]));
+    for (size_t i = 0; i + 1 < S.aptr.size(); ++i) out[19] += S.aptr[i + 1] - S.aptr[i] > 1;
+    out[20] = S.nlevels;
+}
+
 void ldlt_analyze(Handle *h, const int64_t *Puser, const fpsb_ldlt_opts *opts) {
     ldlt_free(h);
     LdltPlan *L = new LdltPlan();
@@ -1096,43 +1184,12 @@ void ldlt_analyze(Handle *h, const int64_t *Puser, const fpsb_ldlt_opts *opts) {
     Symbolic &S = L->S;
     // tasks: big supernodes alone, small ones bundled one per warp
     std::vector<int> tstart, tcnt;
-    {
-        auto small = [&](int s) {
-            int w = S.sfirst[(size_t)s + 1] - S.sfirst[(size_t)s];
-            int nr = (int)(S.rptr[(size_t)s + 1] - S.rptr[(size_t)s]);
-            return w <= kSmallW && (int64_t)w * (w + nr) <= 512;
-        };
-        // `order` is sorted by level: the first nleaf entries are the leaf supernodes; bundles never
-        // straddle the leaf / non-leaf boundary (they are processed by different launches)
-        for (int part = 0; part < 2; part++) {
-            int i = part == 0 ? 0 : S.nleaf;
-            const int end = part == 0 ? S.nleaf : S.nsuper;
-            auto leaf1 = [&](int s) { return part == 0 && S.sfirst[(size_t)s + 1] - S.sfirst[(size_t)s] == 1; };
-            while (i < end) {
-                if (leaf1(S.order[(size_t)i])) { i++; continue; }      // leaf1_*_kernel
-                if (small(S.order[(size_t)i])) {
-                    int j = i;
-                    while (j < end && j - i < kWarpsPerBlock && small(S.order[(size_t)j]) && !leaf1(S.order[(size_t)j])) j++;
-                    tstart.push_back(i); tcnt.push_back(j - i);
-                    i = j;
-                } else {
-                    tstart.push_back(i); tcnt.push_back(0);
-                    i++;
-                }
-            }
-            if (part == 0) L->ntasks_leaf = (int)tstart.size();      // tasks of the leaves wider than one column
-        }
-    }
+    build_tasks(S, tstart, tcnt, L->ntasks_leaf);
     L->ntasks = (int)tstart.size();
     // batched path: one step per dependency level (supernodes of one level do not depend on each other), the CTA-level
     // supernodes of a step first; the one-wide leaves are left to leaf1_factor / leaf1_bwd as in the launches above
     std::vector<int> bsn, bstep;
     {
-        auto warp_level = [&](int t) {
-            const int w = S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t];
-            const int nr = (int)(S.rptr[(size_t)t + 1] - S.rptr[(size_t)t]);
-            return w <= kSmallW && (int64_t)w * (w + nr) <= 512;
-        };
         int i = 0;
         for (int lv = 0; lv < S.nlevels; ++lv) {
             int j = i;
@@ -1142,8 +1199,8 @@ void ldlt_analyze(Handle *h, const int64_t *Puser, const fpsb_ldlt_opts *opts) {
                 if (pass == 1) bstep.push_back((int)bsn.size());
                 for (int k = i; k < j; ++k) {
                     const int t = S.order[(size_t)k];
-                    if (lv == 0 && S.sfirst[(size_t)t + 1] - S.sfirst[(size_t)t] == 1) continue;
-                    if (warp_level(t) == (pass == 1)) bsn.push_back(t);
+                    if (leaf1(S, t)) continue;
+                    if (warp_level(S, t) == (pass == 1)) bsn.push_back(t);
                 }
             }
             bstep.push_back((int)bsn.size());
@@ -1438,6 +1495,11 @@ int fpsb_symbolic_plan_info(fpsb_symbolic s, int64_t *nsuper, int64_t *panel_nnz
     sym_plan(s->S, nsuper, panel_nnz, npairs, flops, nlevels, nleaf);
     return FPSB_OK;
 }
+int fpsb_symbolic_ldlt_routes(fpsb_symbolic s, int64_t out[FPSB_LDLT_ROUTES]) {
+    REQ(s && out, FPSB_EINVAL, "fpsb_symbolic_ldlt_routes: NULL argument");
+    ldlt_routes(s->S, out);
+    return FPSB_OK;
+}
 
 
 
@@ -1517,6 +1579,13 @@ int fpsb_ldlt_plan_info(fpsb_handle hh, int64_t *nsuper, int64_t *panel_nnz, int
     Handle *h = reinterpret_cast<Handle *>(hh);
     REQ(h && h->ldlt, FPSB_ESTATE, "fpsb_ldlt_analyze has not been called");
     sym_plan(h->ldlt->S, nsuper, panel_nnz, npairs, flops, nlevels, nleaf);
+    return FPSB_OK;
+}
+int fpsb_ldlt_routes(fpsb_handle hh, int64_t out[FPSB_LDLT_ROUTES]) {
+    Handle *h = reinterpret_cast<Handle *>(hh);
+    REQ(h && out, FPSB_EINVAL, "fpsb_ldlt_routes: NULL argument");
+    REQ(h->ldlt, FPSB_ESTATE, "fpsb_ldlt_analyze has not been called");
+    ldlt_routes(h->ldlt->S, out);
     return FPSB_OK;
 }
 int fpsb_ldlt_factorize(fpsb_handle hh, double delta, int *factorized) {

@@ -281,6 +281,10 @@ class B200Handle:
         return dict(nsuper=ns.value, panel_nnz=pn.value, npairs=npairs.value, flops=fl.value,
                     nlevels=nl.value, nleaf=nf.value)
 
+    def ldlt_routes(self):
+        """SymbolicAnalysis.routes() of the plan ldlt_analyze built (fpsb_ldlt_routes)."""
+        return _lib.ldlt_routes(_lib.lib().fpsb_ldlt_routes, self.h, "fpsb_ldlt_routes")
+
     def ldlt_factorize(self, delta):
         ok = C.c_int(0)
         check(_lib.lib().fpsb_ldlt_factorize(self.h, C.c_double(delta), C.byref(ok)),

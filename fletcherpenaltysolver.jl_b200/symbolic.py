@@ -43,6 +43,11 @@ class SymbolicAnalysis:
         return dict(nsuper=ns.value, panel_nnz=pn.value, npairs=npairs.value, flops=fl.value,
                     nlevels=nl.value, nleaf=nf.value)
 
+    def routes(self):
+        """Which LDLt routines and staging passes the plan of this analysis goes through (fpsb_symbolic_ldlt_routes;
+        keys: _lib.LDLT_ROUTE_KEYS)."""
+        return _lib.ldlt_routes(_lib.lib().fpsb_symbolic_ldlt_routes, self.h, "fpsb_symbolic_ldlt_routes")
+
     def __del__(self):
         try:
             if self.h:

@@ -200,6 +200,25 @@ int fpsb_symbolic_get(fpsb_symbolic s, int64_t *P, int64_t *parent, int64_t *Lnz
                       int64_t *Li);
 int fpsb_symbolic_plan_info(fpsb_symbolic s, int64_t *nsuper, int64_t *panel_nnz, int64_t *npairs,
                             double *flops, int64_t *nlevels, int64_t *nleaf);
+/* Routes of the supernodal plan through the LDLt kernels, from the predicates the launches use.  Host only.
+ *   [0] supernodes  [1] one-wide leaves (flat leaf kernels)  [2] leaves wider than one column (scalar CTA routines)
+ *   [3] warp-level supernodes (w <= 8 and w (w + nr) <= 512; one-wide leaves excluded)  [4] of those, above the leaves
+ *   [5] warp bundles (tasks of 1..8 warp-level supernodes)  [6] full bundles (8)
+ *   [7] CTA-level supernodes above the leaves (the staged block routines in modes 1 and 2)  [8] of those with w = 64
+ *   [9] of those with 33 <= w <= 63  [10] largest nr (rows below a supernode's diagonal block)
+ *   [11] CTA-level panels (as [7]) with nr > 128 (more than one TRSM pass)  [12] with nr > 1024 (more than one
+ *        backward-solve staging pass)
+ *   update pairs into the supernodes of [7] (Schur update passes), nrow = rows of the source from the pair's first row,
+ *   ncol = its columns in the target, wd = width of the source:
+ *   [13] nrow > 64 (more than one pass)  [14] nrow % 8 != 0  [15] ncol % 8 != 0  [16] wd % 4 != 0
+ *   [17] leaf contributions (leaf_update / leaf_fwd_update entries)  [18] explicit zero slots that relaxed
+ *        amalgamation stores in the lower part of the panels  [19] panel slots assembled from more than one entry
+ *   [20] dependency levels
+ *   last staging pass one row short of full, exactly full, holding one row after a full one: [21..23] TRSM passes of the panels of [7]
+ *   (128 rows), [24..26] backward-solve passes of the same panels (1024 rows), [27..29] Schur update passes of the
+ *   pairs of [13] (64 rows) */
+#define FPSB_LDLT_ROUTES 30
+int fpsb_symbolic_ldlt_routes(fpsb_symbolic s, int64_t out[FPSB_LDLT_ROUTES]);
 
 /* ---------------------------------------------------------------------------------------------
  * LDLt path — LDLtSolver (host symbolic analysis + device numeric refactorisation + 2-RHS solves)
@@ -221,6 +240,8 @@ int fpsb_ldlt_get_symbolic(fpsb_handle h, int64_t *P, int64_t *parent, int64_t *
  * dependency DAG (critical path, in supernodes) and number of leaf supernodes */
 int fpsb_ldlt_plan_info(fpsb_handle h, int64_t *nsuper, int64_t *panel_nnz, int64_t *npairs,
                         double *flops, int64_t *nlevels, int64_t *nleaf);
+/* fpsb_symbolic_ldlt_routes of the plan fpsb_ldlt_analyze built (host only) */
+int fpsb_ldlt_routes(fpsb_handle h, int64_t out[FPSB_LDLT_ROUTES]);
 /* ldl_factorize!(M, str) with vals = [1..1 | jac values | -delta..-delta]
  *   src/solve_linear_system.jl:231-234. Uses the values last given to fpsb_set_jac_values.
  * *factorized mirrors LDLFactorizations.factorized(str). */

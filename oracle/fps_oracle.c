@@ -100,6 +100,7 @@ typedef struct {
     i64 *parent, *Lnz, *Lp, *Li;
     double *Lx, *D, *Y;
     i64 *pattern, *flag;
+    signed char *reg;         /* reg[k] = 1: pivot k was replaced by the dynamic regularisation */
     double r1, r2, tol;
     i64 n_d;
     int factorized;
@@ -110,7 +111,7 @@ void fo_ldl_free(fo_ldl *S)
     if (!S) return;
     free(S->P); free(S->pinv); free(S->Cp); free(S->Ci); free(S->Cpos);
     free(S->parent); free(S->Lnz); free(S->Lp); free(S->Li);
-    free(S->Lx); free(S->D); free(S->Y); free(S->pattern); free(S->flag);
+    free(S->Lx); free(S->D); free(S->Y); free(S->pattern); free(S->flag); free(S->reg);
     free(S);
 }
 
@@ -175,6 +176,7 @@ fo_ldl *fo_ldl_analyze(i64 n, const i64 *Ap, const i64 *Ai, const i64 *P)
     S->Lx = (double *)malloc((size_t)(lnz > 0 ? lnz : 1) * sizeof(double));
     S->D = (double *)calloc((size_t)n, sizeof(double));
     S->Y = (double *)calloc((size_t)n, sizeof(double));
+    S->reg = (signed char *)calloc((size_t)(n > 0 ? n : 1), 1);
     S->factorized = 0;
     return S;
 }
@@ -201,6 +203,9 @@ void fo_ldl_get_numeric(const fo_ldl *S, double *Lx, double *D)
     if (Lx) memcpy(Lx, S->Lx, (size_t)S->Lp[S->n] * sizeof(double));
     if (D) memcpy(D, S->D, (size_t)S->n * sizeof(double));
 }
+
+/* reg[k] = 1 where the last factorisation regularised pivot k (permuted order) */
+void fo_ldl_get_regularised(const fo_ldl *S, signed char *reg) { memcpy(reg, S->reg, (size_t)S->n); }
 
 /* ldl_factorize!(A, S): up-looking LDL' on the permuted matrix; dynamic regularisation.
    Returns 1 when factorised, 0 when a zero pivot was met (S->factorized mirrors it). */
@@ -250,7 +255,8 @@ int fo_ldl_factorize(fo_ldl *S, const i64 *Ap, const i64 *Ai, const double *Ax)
             Lx[p] = l_ki;
             Lnz[i]++;
         }
-        if (dynamic_reg && fabs(D[k]) < S->tol) {
+        S->reg[k] = dynamic_reg && fabs(D[k]) < S->tol;
+        if (S->reg[k]) {
             double r = (S->P[k] < S->n_d) ? S->r1 : S->r2;
             double sgn = (r > 0) - (r < 0);
             double a = fabs(D[k] + r), b = fabs(r);
@@ -1040,4 +1046,173 @@ int fo_ldlt_solve_two_least_squares(fo_ldlt_solver *S, const double *rhs1, const
     memcpy(p2, sol + N, (size_t)nvar * sizeof(double));
     memcpy(q2, sol + N + nvar, (size_t)ncon * sizeof(double));
     return ok;
+}
+
+/* ------------------------------------------------------------------------------------------ */
+/* Error-model checks of a given factor L^, D^ (LDLFactorizations' CSC layout: the Lp / Li of S->str) and of solutions */
+/* computed with it, in long double, against K as the last fo_ldlt_solve_two_mixed assembled it (S->Kp/Ki/Kx).       */
+/* u = 2^-53.  reg (permuted order, may be NULL): pivots replaced by the dynamic regularisation.                      */
+/* ------------------------------------------------------------------------------------------ */
+/* row structure of L: for row i, the columns k < i with L(i, k) structurally nonzero and the position of the value */
+static void ldl_rows(const fo_ldl *L, i64 **Rp_out, i64 **Rpos_out)
+{
+    i64 n = L->n, lnz = L->Lp[n];
+    i64 *Rp = (i64 *)calloc((size_t)n + 1, sizeof(i64));
+    i64 *Rpos = (i64 *)malloc((size_t)(lnz > 0 ? lnz : 1) * sizeof(i64));
+    for (i64 p = 0; p < lnz; p++) Rp[L->Li[p] + 1]++;
+    for (i64 i = 0; i < n; i++) Rp[i + 1] += Rp[i];
+    i64 *w = (i64 *)malloc((size_t)(n + 1) * sizeof(i64));
+    memcpy(w, Rp, (size_t)(n + 1) * sizeof(i64));
+    for (i64 j = 0; j < n; j++)
+        for (i64 p = L->Lp[j]; p < L->Lp[j + 1]; p++) Rpos[w[L->Li[p]]++] = p;   /* ascending column within a row */
+    free(w);
+    *Rp_out = Rp; *Rpos_out = Rpos;
+}
+
+/* diagonal of P K P' (permuted order) */
+static void perm_diag(const fo_ldlt_solver *S, long double *kd)
+{
+    const fo_ldl *L = S->str;
+    for (i64 k = 0; k < S->N; k++) kd[k] = 0.0L;
+    for (i64 c = 0; c < S->N; c++)
+        for (i64 p = S->Kp[c]; p < S->Kp[c + 1]; p++)
+            if (S->Ki[p] == c) kd[L->pinv[c]] += (long double)S->Kx[p];
+}
+
+/* Factor check: for every (i, j) of the pattern of L (diagonal included),
+ *   |(P K P' - L^ D^ L^')_ij| / ((c_ij + 4) u (|L^| |D^| |L^'|)_ij),
+ * c_ij = #{k < j : L(i,k) L(j,k) structurally nonzero}; the diagonal positions of regularised pivots are skipped.
+ * Returns the worst ratio; *where = its position (p < lnz: Lx[p], lnz + j: the diagonal j).  bound (optional, lnz + N):
+ * the denominator of every position.  dpre (optional, N): d_k = (P K P')_kk - sum_{j<k} L^_kj^2 D^_j, the pivot before
+ * any regularisation. */
+double fo_ldlt_check_factor(const fo_ldlt_solver *S, const double *Lx, const double *D, const signed char *reg,
+                            i64 *where, double *bound, double *dpre)
+{
+    const fo_ldl *L = S->str;
+    const i64 n = L->n, lnz = L->Lp[n];
+    const i64 *Lp = L->Lp, *Li = L->Li;
+    const long double u = ldexpl(1.0L, -53);
+    i64 *Rp, *Rpos;
+    ldl_rows(L, &Rp, &Rpos);
+    /* lower triangle of P K P' by permuted columns: (row, value) lists */
+    i64 *Cp = (i64 *)calloc((size_t)n + 1, sizeof(i64));
+    for (i64 c = 0; c < n; c++)
+        for (i64 p = S->Kp[c]; p < S->Kp[c + 1]; p++) {
+            i64 a = L->pinv[S->Ki[p]], b = L->pinv[c];
+            Cp[(a < b ? a : b) + 1]++;
+        }
+    for (i64 j = 0; j < n; j++) Cp[j + 1] += Cp[j];
+    i64 *Ci = (i64 *)malloc((size_t)(Cp[n] > 0 ? Cp[n] : 1) * sizeof(i64));
+    long double *Cx = (long double *)malloc((size_t)(Cp[n] > 0 ? Cp[n] : 1) * sizeof(long double));
+    {
+        i64 *w = (i64 *)malloc((size_t)(n + 1) * sizeof(i64));
+        memcpy(w, Cp, (size_t)(n + 1) * sizeof(i64));
+        for (i64 c = 0; c < n; c++)
+            for (i64 p = S->Kp[c]; p < S->Kp[c + 1]; p++) {
+                i64 a = L->pinv[S->Ki[p]], b = L->pinv[c];
+                i64 q = w[a < b ? a : b]++;
+                Ci[q] = a > b ? a : b; Cx[q] = (long double)S->Kx[p];
+            }
+        free(w);
+    }
+    i64 *col = (i64 *)malloc((size_t)(lnz > 0 ? lnz : 1) * sizeof(i64));
+    for (i64 k = 0; k < n; k++) for (i64 p = Lp[k]; p < Lp[k + 1]; p++) col[p] = k;
+    long double *acc = (long double *)calloc((size_t)(n > 0 ? n : 1), sizeof(long double));
+    long double *mag = (long double *)calloc((size_t)(n > 0 ? n : 1), sizeof(long double));
+    i64 *cnt = (i64 *)calloc((size_t)(n > 0 ? n : 1), sizeof(i64));
+    double worst = 0.0;
+    i64 wpos = -1;
+    for (i64 j = 0; j < n; j++) {
+        /* acc[i] = (L^ D^ L^' - P K P')_ij for i = j and the rows i of column j: the columns k < j of row j contribute
+           their rows from j down (the elimination tree puts them in the pattern of column j) */
+        for (i64 q = Rp[j]; q < Rp[j + 1]; q++) {
+            const i64 pj = Rpos[q], k = col[pj];
+            const long double ljd = (long double)Lx[pj] * (long double)D[k];
+            for (i64 p = pj; p < Lp[k + 1]; p++) {
+                const long double t = (long double)Lx[p] * ljd;
+                acc[Li[p]] += t; mag[Li[p]] += fabsl(t); cnt[Li[p]]++;
+            }
+        }
+        acc[j] += (long double)D[j]; mag[j] += fabsl((long double)D[j]);      /* k = j, L(j, j) = 1 */
+        for (i64 p = Lp[j]; p < Lp[j + 1]; p++) {
+            const long double t = (long double)Lx[p] * (long double)D[j];
+            acc[Li[p]] += t; mag[Li[p]] += fabsl(t);
+        }
+        for (i64 p = Cp[j]; p < Cp[j + 1]; p++) acc[Ci[p]] -= Cx[p];
+        if (dpre) dpre[j] = (double)((long double)D[j] - acc[j]);
+        for (i64 e = -1; e < Lp[j + 1] - Lp[j]; e++) {
+            const i64 i = e < 0 ? j : Li[Lp[j] + e];
+            const i64 pos = e < 0 ? lnz + j : Lp[j] + e;
+            const long double b = (long double)(cnt[i] + 4) * u * mag[i];
+            if (bound) bound[pos] = (double)b;
+            if (!(e < 0 && reg && reg[j])) {
+                const long double err = fabsl(acc[i]);
+                const double r = err == 0.0L ? 0.0 : (b > 0.0L ? (double)(err / b) : INFINITY);
+                if (wpos < 0 || r > worst) { worst = r; wpos = pos; }
+            }
+            acc[i] = 0.0L; mag[i] = 0.0L; cnt[i] = 0;
+        }
+    }
+    if (where) *where = wpos;
+    free(Rp); free(Rpos); free(Cp); free(Ci); free(Cx); free(acc); free(mag); free(cnt); free(col);
+    return worst;
+}
+
+/* Solve check of one solution x^ (original order, N) of K x = b: for every i,
+ *   |b - K~ x^|_i / ((3c + 10) u (P' |L^| |D^| |L^'| P |x^|)_i),
+ * c = the largest row or column count of L, K~ = K with the pivot change D^_k - d_k (fo_ldlt_check_factor's dpre) added
+ * at the regularised positions k, whose factor is the one L^ D^ L^' stands for.  Returns the worst ratio, *where = i. */
+double fo_ldlt_check_solve(const fo_ldlt_solver *S, const double *Lx, const double *D, const signed char *reg,
+                           const double *x, const double *b, i64 *where)
+{
+    const fo_ldl *L = S->str;
+    const i64 n = L->n;
+    const i64 *Lp = L->Lp, *Li = L->Li, *P = L->P;
+    const long double u = ldexpl(1.0L, -53);
+    long double *y = (long double *)calloc((size_t)(n > 0 ? n : 1), sizeof(long double));
+    long double *t = (long double *)calloc((size_t)(n > 0 ? n : 1), sizeof(long double));
+    long double *t3 = (long double *)calloc((size_t)(n > 0 ? n : 1), sizeof(long double));
+    i64 *rc = (i64 *)calloc((size_t)(n > 0 ? n : 1), sizeof(i64));
+    i64 c = 0;
+    for (i64 j = 0; j < n; j++) {
+        i64 cc = Lp[j + 1] - Lp[j];
+        if (cc > c) c = cc;
+        for (i64 p = Lp[j]; p < Lp[j + 1]; p++) rc[Li[p]]++;
+    }
+    for (i64 i = 0; i < n; i++) if (rc[i] > c) c = rc[i];
+    /* K x (K holds the upper triangle) */
+    for (i64 col = 0; col < n; col++)
+        for (i64 p = S->Kp[col]; p < S->Kp[col + 1]; p++) {
+            const i64 r = S->Ki[p];
+            const long double v = (long double)S->Kx[p];
+            y[r] += v * (long double)x[col];
+            if (r != col) y[col] += v * (long double)x[r];
+        }
+    if (reg) {
+        /* d_k = (P K P')_kk - sum_j L^_kj^2 D^_j */
+        perm_diag(S, t);
+        for (i64 j = 0; j < n; j++)
+            for (i64 p = Lp[j]; p < Lp[j + 1]; p++) t[Li[p]] -= (long double)Lx[p] * (long double)Lx[p] * (long double)D[j];
+        for (i64 k = 0; k < n; k++)
+            if (reg[k]) y[P[k]] += ((long double)D[k] - t[k]) * (long double)x[P[k]];
+    }
+    /* P' |L^| |D^| |L^'| P |x^|: t = |L^'| z, t *= |D^|, t3 = |L^| t */
+    for (i64 k = 0; k < n; k++) t[k] = fabsl((long double)x[P[k]]);
+    for (i64 j = 0; j < n; j++)
+        for (i64 p = Lp[j]; p < Lp[j + 1]; p++) t[j] += fabsl((long double)Lx[p]) * fabsl((long double)x[P[Li[p]]]);
+    for (i64 k = 0; k < n; k++) { t[k] *= fabsl((long double)D[k]); t3[k] = t[k]; }
+    for (i64 j = 0; j < n; j++)
+        for (i64 p = Lp[j]; p < Lp[j + 1]; p++) t3[Li[p]] += fabsl((long double)Lx[p]) * t[j];
+    double worst = 0.0;
+    i64 wi = -1;
+    for (i64 k = 0; k < n; k++) {
+        const i64 i = P[k];
+        const long double err = fabsl((long double)b[i] - y[i]);
+        const long double bd = (long double)(3 * c + 10) * u * t3[k];
+        const double r = err == 0.0L ? 0.0 : (bd > 0.0L ? (double)(err / bd) : INFINITY);
+        if (wi < 0 || r > worst) { worst = r; wi = i; }
+    }
+    if (where) *where = wi;
+    free(y); free(t); free(t3); free(rc);
+    return worst;
 }

@@ -95,6 +95,8 @@ def lib():
         _lib.fo_ldl_n.restype = C.c_int64
         _lib.fo_ldl_lnz.restype = C.c_int64
         _lib.fo_coo_to_csc.restype = C.c_int64
+        _lib.fo_ldlt_check_factor.restype = C.c_double
+        _lib.fo_ldlt_check_solve.restype = C.c_double
     return _lib
 
 
@@ -159,6 +161,12 @@ class LDL:
         Lx = np.zeros(max(lnz, 1)); D = np.zeros(self.n)
         lib().fo_ldl_get_numeric(self.h, _p(Lx), _p(D))
         return Lx[:lnz], D
+
+    def regularised(self):
+        """Boolean mask (permuted order) of the pivots the last factorisation regularised."""
+        reg = np.zeros(self.n, np.int8)
+        lib().fo_ldl_get_regularised(self.h, _p(reg))
+        return reg.astype(bool)
 
     def __del__(self):
         try:
@@ -295,6 +303,32 @@ class LDLtOracle:
 
     def numeric(self):
         return self._str().numeric()
+
+    def regularised(self):
+        return self._str().regularised()
+
+    def check_factor(self, Lx, D, reg=None):
+        """Per-entry error-model check of a factor L^, D^ in this oracle's CSC layout against K as the last
+        solve_two_mixed assembled it, in long double: max over the pattern of L (diagonal included, the diagonals of
+        the `reg` pivots skipped) of |(P K P' - L^ D^ L^')_ij| / ((c_ij + 4) 2^-53 (|L^| |D^| |L^'|)_ij), c_ij the
+        number of k < j with L(i,k) L(j,k) structurally nonzero.  Returns dict(ratio, where, bound, dpre): `where`
+        indexes [Lx | D], `bound` holds every denominator, `dpre` the pivots before regularisation."""
+        Lx, D = _f64(Lx), _f64(D)
+        N = self.nvar + self.ncon
+        reg = None if reg is None else np.ascontiguousarray(reg, dtype=np.int8)
+        bound = np.zeros(len(Lx) + N); dpre = np.zeros(N); where = C.c_int64(-1)
+        r = lib().fo_ldlt_check_factor(self.h, _p(Lx), _p(D), _p(reg), C.byref(where), _p(bound), _p(dpre))
+        return dict(ratio=r, where=where.value, bound=bound, dpre=dpre)
+
+    def check_solve(self, Lx, D, x, b, reg=None):
+        """Error-model check of a solution x^ = [p; q] of K x = b computed with L^, D^, in long double: max over i of
+        |b - K~ x^|_i / ((3c + 10) 2^-53 (P' |L^| |D^| |L^'| P |x^|)_i), c the largest row or column count of L,
+        K~ = K plus the pivot changes of the `reg` pivots.  Returns (ratio, i)."""
+        Lx, D, x, b = _f64(Lx), _f64(D), _f64(x), _f64(b)
+        reg = None if reg is None else np.ascontiguousarray(reg, dtype=np.int8)
+        where = C.c_int64(-1)
+        r = lib().fo_ldlt_check_solve(self.h, _p(Lx), _p(D), _p(reg), _p(x), _p(b), C.byref(where))
+        return r, where.value
 
     def solve_two_mixed(self, jvals, delta, rhs1, rhs2):
         jvals, rhs1, rhs2 = _f64(jvals), _f64(rhs1), _f64(rhs2)

@@ -72,6 +72,18 @@ def test_tile_layout_and_create_validation():
     assert rc == -1 and b"out of range" in L.fpsb_last_error()
 
 
+def test_ldlt_routes_validation():
+    """fpsb_symbolic_ldlt_routes and fpsb_ldlt_routes reject a NULL analysis / handle and a NULL output."""
+    L = _lib.lib()
+    out = (ctypes.c_int64 * len(_lib.LDLT_ROUTE_KEYS))()
+    assert L.fpsb_symbolic_ldlt_routes(None, out) == -1 and b"NULL" in L.fpsb_last_error()
+    assert L.fpsb_ldlt_routes(None, out) == -1 and b"NULL" in L.fpsb_last_error()
+    S = SymbolicAnalysis(3, 2, [0, 1], [0, 2])
+    assert L.fpsb_symbolic_ldlt_routes(S.h, None) == -1
+    rt = S.routes()
+    assert rt["nsuper"] >= 1 and rt["leaf1"] + rt["leaf_wide"] >= 1
+
+
 @pytest.mark.parametrize("m,n,k,w", [(1, 10, 9, 4), (30, 60, 5, 8), (500, 1000, 10, 32), (4000, 8000, 10, 64)])
 @pytest.mark.parametrize("pk", ["amd", "id", "rand"])
 def test_symbolic_bit_exact_vs_oracle(oracle, m, n, k, w, pk):
